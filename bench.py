@@ -2,6 +2,7 @@
 """bench.py -- factor-aggregation edges/s (fwd+bwd) and link-pair scores/s on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c5|c6|c4|c4k5|c4k5d64|mid|tiny] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole graph and pair batch:
     attention -> aggregation -> pair scoring -> BCE gradient -> decoder backward -> factor backward
@@ -613,6 +614,27 @@ def gen_pairs_from_edges(src, dst, N, E, P, dev):
 PHASES = ["wait", "ag_Z", "attn_fwd", "ag_s", "spmm_fwd", "ag_H", "pair_fwd", "ag_prob", "loss", "pair_bwd",
           "ag_dH", "bwd_gather", "ag_r", "bwd_edges"]
 KERNEL_PHASES = ["attn_fwd", "spmm_fwd", "pair_fwd", "pair_bwd", "bwd_gather", "bwd_edges"]
+DUMP_PAIRS = 1 << 20     # sampled link scores
+DUMP_ROWS = 1 << 14      # sampled node rows of H and dL/dZ (K*d floats each): 20 MB in all at K*d = 128
+
+
+def dump_outputs(out_dir, step):
+    """What the last timed step handed its caller, as float .npy files in out_dir: loss [1] (float64),
+    prob [<= DUMP_PAIRS] (link scores), H and dZ [<= DUMP_ROWS, K, d] (embeddings and dL/dZ of the
+    nodes).  Larger outputs are sampled at indices drawn from a fixed seed, so two builds run with the
+    same arguments dump the same entries."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    pick = lambda n, k: torch.from_numpy(np.sort(rng.choice(n, size=min(n, k), replace=False))).to(step.device)
+    pairs, rows = pick(step.P, DUMP_PAIRS), pick(step.n_own, DUMP_ROWS)
+    out = {"loss": np.array([float(step.loss.item())], dtype=np.float64),
+           "prob": step.prob[:step.P][pairs].cpu().numpy(),
+           "H": step.H[:step.n_own][rows].cpu().numpy(),
+           "dZ": step.dZ[rows].cpu().numpy()}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_native(args):
@@ -696,6 +718,8 @@ def run_native(args):
     torch.cuda.profiler.stop()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, step)
     abi_calls = _lib.launches - launches0
     total_ms = ev_a.elapsed_time(ev_b)
     # per-phase times from consecutive events
@@ -1055,7 +1079,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the comparison with a single-GPU step")
     ap.add_argument("--no-configs", action="store_true", help="skip the side measurements of BASELINE configs[0..3]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's loss, scores, H and dL/dZ (seeded samples) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "native" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs: native arm on one GPU only")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,10 +1,16 @@
-"""The CPU oracle against the UNMODIFIED reference, live: baseline/_ref/model.py (a byte-for-byte copy
-staged by tools/stage_reference.sh; git-ignored, travels to the GPU box) is imported as is and driven
-through its own Disentangle.forward (model.py:105-114) on seeded random graphs that the committed
-fixtures do not hold -- duplicate edge columns, self-loops, isolated nodes, K = 1, K > 8, T != 1,
-beta at both ends -- and the oracle has to reproduce adj_sym.nonzero() bit for bit and routing, softmax
-weights, row sums, embeddings, ALL N^2 link scores and dL/dZ of a BCE over all N^2 scores within the
-north_star tolerance (1e-5 relative).  Skipped when the staged copy is absent.
+"""The CPU oracle against the reference's dense math on seeded random graphs that the committed fixtures
+do not hold -- duplicate edge columns, self-loops, isolated nodes, K = 1, K > 8, T != 1, beta at both
+ends.  The oracle has to reproduce adj_sym.nonzero() bit for bit and routing, softmax weights, row sums,
+embeddings, ALL N^2 link scores and dL/dZ of a BCE over all N^2 scores within the north_star tolerance
+(1e-5 relative).
+
+Two sources of the dense side, same cases, same assertions:
+  * `dense_layer` below, a line-by-line restatement of Disentangle_layer.forward / Disentangle.forward
+    (model.py:56-77, 105-114).  It is pinned to the UNMODIFIED reference by the committed golden vectors
+    (tests/golden/tiny_*.npz, produced by make_golden.py from model.py as is): it must reproduce their H,
+    N^2 link scores, script loss and dL/dZ.  Runs everywhere.
+  * live: baseline/_ref/model.py (a byte-for-byte copy staged by tools/stage_reference.sh; git-ignored)
+    imported as is and driven through its own Disentangle.forward.  Skipped when the staged copy is absent.
 """
 import importlib.util
 import os
@@ -15,13 +21,13 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from conftest import ROOT
+from conftest import ROOT, load_golden
 
 REF_MODEL = os.path.join(ROOT, "baseline", "_ref", "model.py")
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_MODEL), reason="baseline/_ref/model.py not staged")
 
 RTOL = 1e-5
 TIE_MARGIN = 1e-5
+PIN_RTOL = 1e-6          # restatement vs the reference's stored outputs (bit-equal where the BLAS is the same)
 
 
 @pytest.fixture(scope="module")
@@ -43,6 +49,29 @@ class _Leaf(nn.Module):
         return self.z
 
 
+def dense_layer(Z, adj, beta, T):
+    """Disentangle_layer.forward (model.py:56-77) on a list of K [N,d] tensors -> (h_list, alpha0, att)."""
+    alpha0 = torch.stack([torch.exp(torch.mm(z, z.t()) / T) for z in Z])     # :56-57
+    alpha = alpha0 / torch.sum(alpha0, dim=0)                                  # :59-60
+    p_adj = (torch.argmax(alpha, dim=0) + 1) * adj                             # :61-62 (first max wins)
+    h_list, att = [], []
+    for k, z in enumerate(Z):
+        a1 = (p_adj == k + 1).float() * alpha[k]                                # :64-69
+        s = torch.sum(a1, dim=1)
+        s[s == 0] = 1
+        a1 = a1 / s                                                             # divides column j by s[j]
+        att.append(a1)
+        h_list.append(beta * z + (1 - beta) * torch.mm(a1, z))                 # :75
+    return h_list, alpha0, att
+
+
+def dense_forward(Z, adj, beta, T):
+    """Disentangle.forward after the factor MLPs (model.py:107-114) -> (alpha0, att, H [N,K*d], link_pred)."""
+    h_list, alpha0, att = dense_layer(Z, adj, beta, T)
+    link_pred = torch.sigmoid(sum(torch.mm(h, h.t()) * a for h, a in zip(h_list, alpha0)))
+    return alpha0, att, torch.cat(h_list, dim=1), link_pred
+
+
 def relerr(a, b):
     a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30)) if b.size else 0.0
@@ -56,6 +85,12 @@ def adj_sym_of(src, dst, n):
     a = adj + adj.t()
     a[a != 0] = 1
     return a
+
+
+def dense_mask(u, v, n):
+    """main_disentangled.py:167-178 (duplicates SUM)"""
+    ei = torch.stack([torch.as_tensor(u), torch.as_tensor(v)])
+    return torch.sparse_coo_tensor(ei, torch.ones(ei.shape[1]), torch.Size([n, n])).to_dense()
 
 
 def make_case(seed):
@@ -76,21 +111,33 @@ def make_case(seed):
     return n, K, d, beta, T, src.astype(np.int64), dst.astype(np.int64), Z
 
 
-@pytest.mark.parametrize("seed", range(48))
-def test_oracle_matches_live_reference(oracle, refmodel, seed):
+def live_reference(refmodel):
+    def run(n, K, d, beta, T, Z, adj, target):
+        m = refmodel.Disentangle(3, 2, d, nfactor=K, beta=beta, t=T)
+        m.factors = [_Leaf(torch.from_numpy(Z[:, k, :].copy())) for k in range(K)]   # a plain list in the reference (model.py:94-97)
+        zs = [f(None) for f in m.factors]
+        _, alpha0, att = m.disentangle_layer1(zs, adj)
+        H_ref, link_pred = m(torch.zeros(n, 3), adj)
+        loss = F.binary_cross_entropy(link_pred, target)
+        loss.backward()
+        return alpha0.detach(), att, H_ref, link_pred, float(loss.detach()), np.stack([f.z.grad.numpy() for f in m.factors], 1)
+    return run
+
+
+def restated_reference(n, K, d, beta, T, Z, adj, target):
+    zs = [torch.from_numpy(Z[:, k, :].copy()).requires_grad_(True) for k in range(K)]
+    alpha0, att, H_ref, link_pred = dense_forward(zs, adj, beta, T)
+    loss = F.binary_cross_entropy(link_pred, target)
+    loss.backward()
+    return alpha0.detach(), att, H_ref, link_pred, float(loss.detach()), np.stack([z.grad.numpy() for z in zs], 1)
+
+
+def check_case(oracle, seed, reference):
     torch.set_num_threads(4)
     n, K, d, beta, T, src, dst, Z = make_case(seed)
     adj = adj_sym_of(src, dst, n)
-    m = refmodel.Disentangle(3, 2, d, nfactor=K, beta=beta, t=T)
-    m.factors = [_Leaf(torch.from_numpy(Z[:, k, :].copy())) for k in range(K)]   # a plain list in the reference (model.py:94-97)
-    zs = [f(None) for f in m.factors]
-    h_list, alpha0, att = m.disentangle_layer1(zs, adj)
-    H_ref, link_pred = m(torch.zeros(n, 3), adj)
     target = (torch.from_numpy(np.random.default_rng(seed).random((n, n))) < 0.3).float()
-    loss = F.binary_cross_entropy(link_pred, target)
-    loss.backward()
-    ref_loss = float(loss.detach())
-    dZ_ref = np.stack([f.z.grad.numpy() for f in m.factors], 1)
+    e_ref, att, H_ref, link_pred, ref_loss, dZ_ref = reference(n, K, d, beta, T, Z, adj, target)
 
     # integer structure: bit-exact
     rowptr, col = oracle.csr_from_edges(src, dst, n)
@@ -100,8 +147,7 @@ def test_oracle_matches_live_reference(oracle, refmodel, seed):
 
     # routing / softmax weight / att / row sums on the CSR entries (model.py:56-74)
     H, ks, w, s = oracle.factor_fwd(rowptr, col, Z, beta, T)
-    e_ref = alpha0.detach()                                   # alpha0 = exp(q) [K,N,N]; the softmax is alpha0 / sum_k
-    a_ref = (e_ref / e_ref.sum(0)).numpy()[:, rows, col]      # model.py:59-60, [K, nnz]
+    a_ref = (e_ref / e_ref.sum(0)).numpy()[:, rows, col]      # alpha0 = exp(q) [K,N,N]; model.py:59-60, [K, nnz]
     ks_ref = a_ref.argmax(0)
     top = np.sort(a_ref, 0)
     margin = top[-1] - top[-2] if K > 1 else np.ones(ks_ref.size)
@@ -125,3 +171,36 @@ def test_oracle_matches_live_reference(oracle, refmodel, seed):
     dZ_dec, dH = oracle.pair_score_bwd(uu, vv, Z, H, dS, T)
     dZ = oracle.factor_bwd(rowptr, col, Z, dH, ks, w, s, beta, T, dZ_init=dZ_dec)
     assert relerr(dZ, dZ_ref) < 5 * RTOL
+
+
+@pytest.mark.parametrize("name", ["tiny_generic", "tiny_deadfactor_T2", "tiny_ties", "tiny_K1", "tiny_empty"])
+def test_restatement_reproduces_the_reference_outputs(name):
+    """dense_layer / dense_forward against what the unmodified model.py computed on the committed tiny fixtures
+    (ties, a factor that never wins, K = 1, T = 2, an empty graph): all N^2 link scores, H, and -- where the fixture
+    holds them -- the script's loss (main_disentangled.py:195) and dL/dZ."""
+    g = load_golden(name)
+    n, K = int(g["N"]), int(g["K"])
+    zs = [torch.from_numpy(g["Z"][:, k, :].copy()).requires_grad_(True) for k in range(K)]
+    _, _, H, link_pred = dense_forward(zs, adj_sym_of(g["src"], g["dst"], n), float(g["beta"]), float(g["T"]))
+    assert relerr(H.detach().numpy(), g["ref_H"]) < PIN_RTOL
+    assert relerr(link_pred.detach().numpy(), g["ref_link_pred"]) < PIN_RTOL
+    if "ref_dZ" in g:
+        ones = torch.ones(n, n)
+        pos = dense_mask(g["loss_pos_u"], g["loss_pos_v"], n)
+        neg = dense_mask(g["loss_neg_u"], g["loss_neg_v"], n)
+        loss = F.binary_cross_entropy(link_pred[pos == 1].unsqueeze(0), ones[pos == 1].unsqueeze(0)) + \
+            F.binary_cross_entropy(link_pred[neg == 1].unsqueeze(0), torch.zeros_like(ones[neg == 1]).unsqueeze(0)) / int(g["m"])
+        loss.backward()
+        assert abs(loss.item() - float(g["ref_loss"])) <= PIN_RTOL * abs(float(g["ref_loss"]))
+        assert relerr(np.stack([z.grad.numpy() for z in zs], 1), g["ref_dZ"]) < PIN_RTOL
+
+
+@pytest.mark.parametrize("seed", range(48))
+def test_oracle_matches_restated_reference(oracle, seed):
+    check_case(oracle, seed, restated_reference)
+
+
+@pytest.mark.skipif(not os.path.exists(REF_MODEL), reason="baseline/_ref/model.py not staged")
+@pytest.mark.parametrize("seed", range(48))
+def test_oracle_matches_live_reference(oracle, refmodel, seed):
+    check_case(oracle, seed, live_reference(refmodel))

@@ -4,11 +4,6 @@
 # (load with DL_LIB_PATH=disenlink_b200/_variants/lib_NAME.so; the other objects come from the regular build)
 set -e
 cd "$(dirname "$0")/.."
-name=$1; src=$2; shift 2
-mkdir -p disenlink_b200/_variants
-obj=disenlink_b200/_variants/${name}_$(basename ${src%.cu}).o
-/usr/local/cuda/bin/nvcc -ccbin /usr/bin/g++ -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 \
-  --fmad=false -Xcompiler -fPIC -Xptxas -v "$@" -c disenlink_b200/csrc/$src -o $obj 2> disenlink_b200/_variants/${name}.ptxas.log
-others=$(ls disenlink_b200/_obj/*.o | grep -v "/$(basename ${src%.cu}).o")
-/usr/local/cuda/bin/nvcc -ccbin /usr/bin/g++ -shared -o disenlink_b200/_variants/lib_${name}.so $obj $others -lcudart -Xlinker -z -Xlinker defs
+name=$1
+python -m disenlink_b200.build --variant "$@"
 grep -A2 "flILi8ELi16\|Li8, *Li16\|ILi8ELi16" disenlink_b200/_variants/${name}.ptxas.log | grep -E "spill|Used" | head -4
