@@ -23,8 +23,9 @@ DL_HUB_BUCKET_END = 23
 # dl_graph.flags (kernel-path switches for A/B runs and for testing the non-default paths)
 DL_F_NO_STREAM, DL_F_NO_FL, DL_F_NO_FL_ATTN, DL_F_NO_PRESCALE = 1, 2, 4, 8
 DL_F_NO_SJ, DL_F_NO_SR, DL_F_NO_XDOT, DL_F_NO_SYM = 16, 32, 64, 128
+DL_F_NO_KEEPA = 256
 _FLAG_NAMES = {"NO_STREAM": 1, "NO_FL": 2, "NO_FL_ATTN": 4, "NO_PRESCALE": 8, "NO_SJ": 16, "NO_SR": 32,
-               "NO_XDOT": 64, "NO_SYM": 128}
+               "NO_XDOT": 64, "NO_SYM": 128, "NO_KEEPA": 256}
 DL_EASYM, DL_EUNSUPPORTED = -4, -5
 
 
@@ -78,13 +79,13 @@ SIGNATURES = {
     "dl_edge_attn_fwd": (_int, [_GP, _vp, _int, _int, _f, _vp, _vp, _vp, _vp, _vp]),
     "dl_sym_index_workspace_bytes": (_sz, [_i64, _i64]),
     "dl_sym_index": (_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
-    "dl_edge_attn_fwd_sym": (_int, [_GP, _GP, _vp, _vp, _int, _int, _f, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dl_edge_attn_fwd_sym": (_int, [_GP, _GP, _vp, _vp, _int, _int, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "dl_factor_spmm_fwd": (_int, [_GP, _vp, _vp, _vp, _vp, _int, _int, _f, _f, _vp, _vp, _vp, _i64, _vp, _vp]),
     "dl_factor_bwd": (_int, [_GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _int, _int, _f, _f, _f, _vp, _vp, _vp, _vp]),
     "dl_factor_bwd_gather": (_int, [_GP, _vp, _vp, _vp, _vp, _vp, _int, _int, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "dl_factor_bwd_edges_sym_supported": (_int, [_int, _int]),
-    "dl_factor_bwd_edges_sym": (_int, [_GP, _GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _int, _int, _f, _f, _vp,
-                                       _vp, _vp]),
+    "dl_factor_bwd_edges_sym": (_int, [_GP, _GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _int, _int, _f, _f, _int,
+                                       _vp, _vp, _vp]),
     "dl_factor_bwd_edges": (_int, [_GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _int, _int, _f, _f, _vp, _vp, _vp]),
     "dl_pair_score_fwd": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _int, _int, _f, _vp, _vp, _vp]),
     "dl_pair_incidence_workspace_bytes": (_sz, [_i64, _i64]),

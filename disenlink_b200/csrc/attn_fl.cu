@@ -78,9 +78,11 @@ __device__ __forceinline__ float afl_dot(const float4 (&a)[C::C4], const float4 
 template <int K_, int d_>
 __global__ void __launch_bounds__(AflCfg<K_, d_>::THREADS, 1)
 k_attn_fl(DlGraphDev g, const float* __restrict__ Z, float T, unsigned char* __restrict__ kstar,
-          float* __restrict__ w, float* __restrict__ s, float* __restrict__ carry, float2* __restrict__ kw_out) {
+          float* __restrict__ w, float* __restrict__ s, float* __restrict__ carry, float2* __restrict__ kw_out,
+          float* __restrict__ a_out) {
   // kw_out != nullptr (symmetric attention, attn_sym.cu): g is the UPPER-triangle view of the graph; the
-  // routing of entry e goes to kw_out[e] = (w, kstar) as one 8-byte record and no row sums are made here
+  // routing of entry e goes to kw_out[e] = (w, kstar) as one 8-byte record and no row sums are made here.
+  // a_out != nullptr (only with kw_out): the softmax of entry e goes to a_out[e * K + kap] for backward pass 2
   using C = AflCfg<K_, d_>;
   constexpr int K = C::K, d = C::d, D = C::D, LPE = C::LPE, EPS = C::EPS, QPC = C::QPC, C4 = C::C4;
   constexpr int ROWS = C::ROWS, STAGE_B = C::STAGE_B;
@@ -266,6 +268,7 @@ k_attn_fl(DlGraphDev g, const float* __restrict__ Z, float T, unsigned char* __r
         const unsigned hit = __ballot_sync(DL_FULL, key == mx && factive);
         const int ks = __ffs((hit >> gbase) & 0xffu) - 1;
         const float wv = __shfl_sync(DL_FULL, a, gbase + ks);
+        if (a_out && valid && factive) a_out[(c * DL_CH + src) * K + kap] = a;   // 4K contiguous bytes per entry
         if (valid && kap == 0) {
           const long long e = c * DL_CH + src;
           if (kw_out) {
@@ -304,7 +307,7 @@ k_attn_fl(DlGraphDev g, const float* __restrict__ Z, float T, unsigned char* __r
 template <int K_, int d_>
 struct AflLaunch {
   static int run(const DlGraphDev& g, const float* Z, float T, unsigned char* kstar, float* w, float* s,
-                 float* carry, float2* kw_out, cudaStream_t st) {
+                 float* carry, float2* kw_out, float* a_out, cudaStream_t st) {
     using C = AflCfg<K_, d_>;
     int dev = 0, sms = 0;
     DL_CUDA_TRY(cudaGetDevice(&dev));
@@ -316,7 +319,7 @@ struct AflLaunch {
     long long grid = (n_ranges + C::NW - 1) / C::NW;
     if (grid > sms) grid = sms;
     if (grid < 1) grid = 1;
-    k_attn_fl<K_, d_><<<(int)grid, C::THREADS, C::SMEM, st>>>(g, Z, T, kstar, w, s, carry, kw_out);
+    k_attn_fl<K_, d_><<<(int)grid, C::THREADS, C::SMEM, st>>>(g, Z, T, kstar, w, s, carry, kw_out, a_out);
     DL_LAUNCH_CHECK();
     return DL_OK;
   }
@@ -325,14 +328,16 @@ struct AflLaunch {
 }  // namespace
 
 // returns -1000 when (K, d) has no factor-per-lane instantiation; scratch: 3 * n_ranges * K floats.
-// kw_out != nullptr: packed (w, kstar) records, no row sums (kstar, w, s, scratch may be null)
+// kw_out != nullptr: packed (w, kstar) records, no row sums (kstar, w, s, scratch may be null); a_out (only
+// with kw_out, may be null): the softmax a [nnz, K]
 int dl_launch_attn_fl(const DlGraphDev& g, const float* Z, int K, int d, float T, unsigned char* kstar,
-                      float* w, float* s, float* scratch, cudaStream_t st, float2* kw_out) {
+                      float* w, float* s, float* scratch, cudaStream_t st, float2* kw_out, float* a_out) {
   if (!g.erow || g.nnz == 0 || (!scratch && !kw_out)) return -1000;
   if (kw_out) s = nullptr;
+  else a_out = nullptr;
   int rc = -1000;
 #define AFL_CASE(KK, DD) \
-  if (K == KK && d == DD) rc = AflLaunch<KK, DD>::run(g, Z, T, kstar, w, s, scratch, kw_out, st);
+  if (K == KK && d == DD) rc = AflLaunch<KK, DD>::run(g, Z, T, kstar, w, s, scratch, kw_out, a_out, st);
   AFL_CASE(8, 16)
   AFL_CASE(8, 8)
   AFL_CASE(5, 16)

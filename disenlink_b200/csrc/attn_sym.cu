@@ -11,7 +11,8 @@
 //      entry e of the full CSR, eidx[e] = its position in the primary view, or ~(its mirror's position)
 //      for a secondary entry.  ("upper" / "lower" in names = primary / secondary.)
 //   2. k_attn_fl on the upper view: one row gather per undirected edge, result written as one packed
-//      8-byte record kw[t] = (w, kstar) per upper entry (coalesced).
+//      8-byte record kw[t] = (w, kstar) per upper entry (coalesced); optionally also the softmax a[t, :]
+//      (4K bytes per upper entry, coalesced), which backward pass 2 then reads instead of recomputing it.
 //   3. k_sym_expand (this file): a streaming pass over the full CSR that reads kw[eidx[e]] -- sequential
 //      for the upper entries of a row, one random 8-byte access for the lower ones --, writes kstar[e]
 //      and w[e] in the layout every other kernel reads, and makes the routed row sums s[i,k] in CSR
@@ -263,7 +264,7 @@ int dl_sym_index(const int64_t* rowptr, const int32_t* col, const int32_t* erow,
 
 int dl_edge_attn_fwd_sym(const dl_graph* g_host, const dl_graph* upper_host, const int32_t* eidx, const float* Z,
                          int K, int d, float T, uint8_t* kstar, float* w, float* s, float* hub_ws, float* kw_scratch,
-                         dl_stream_t stream) {
+                         float* a_out, dl_stream_t stream) {
   if (!dl_graph_ok(g_host) || !dl_graph_ok(upper_host) || !dl_shape_ok(K, d)) return DL_EINVAL;
   if (g_host->N == 0) return DL_OK;
   if (g_host->row_base != 0 || upper_host->row_base != 0 || upper_host->N != g_host->N) return DL_EINVAL;
@@ -275,7 +276,8 @@ int dl_edge_attn_fwd_sym(const dl_graph* g_host, const dl_graph* upper_host, con
   const DlGraphDev g = dl_graph_dev(g_host);
   const DlGraphDev gu = dl_graph_dev(upper_host);
   float2* kw = reinterpret_cast<float2*>(kw_scratch);
-  int rc = dl_launch_attn_fl(gu, Z, K, d, T, nullptr, nullptr, nullptr, nullptr, st, kw);
+  if (g_host->flags & DL_F_NO_KEEPA) a_out = nullptr;
+  int rc = dl_launch_attn_fl(gu, Z, K, d, T, nullptr, nullptr, nullptr, nullptr, st, kw, a_out);
   if (rc == -1000) return DL_EUNSUPPORTED;
   if (rc) return rc;
   int dev = 0, sms = 0;

@@ -47,6 +47,12 @@ namespace {
 #ifndef FL_RING_X
 #define FL_RING_X 2
 #endif
+#ifndef FL_RING_A
+#define FL_RING_A 3
+#endif
+#ifndef FL_MAXW_A
+#define FL_MAXW_A 16
+#endif
 constexpr int FL_OWN = FL_OWN_N;     // staged own-row slots per stage; further rows of a step are read with plain loads
 
 // MODE 0: the routed slice G[j,k*] is staged and <G[j,k*], Z[i,k*]> computed here;
@@ -54,10 +60,16 @@ constexpr int FL_OWN = FL_OWN_N;     // staged own-row slots per stage; further 
 // MODE 2 (symmetric pass 2, phase A, see bwd_sym.cu): MODE 1 on the UPPER-triangle view of the graph
 //        (kstar and x in upper-view order, left there by pass 1), and the K coefficients of every entry
 //        are stored for the lower-triangle phase
+// MODE 3 (KEEPA): MODE 2 with the softmax a[e, :] the symmetric attention stored in coef_out (same layout):
+//        a is staged with the neighbour rows and overwritten in place by the coefficients, so neither the
+//        own row Z[i] nor the K dots, exponentials and the softmax sum are needed here
 template <int K_, int d_, int MODE>
 struct FlCfg {
   static constexpr bool HAS_X = MODE >= 1;
-  static constexpr int FL_RING = HAS_X ? FL_RING_X : FL_RING_N;   // stages per warp ring (FL_RING - 1 in flight)
+  static constexpr bool KEEPA = MODE == 3;
+  // stages per warp ring (FL_RING - 1 in flight); KEEPA stages are ~0.8x the size, which leaves room for one
+  // more stage in flight
+  static constexpr int FL_RING = KEEPA ? FL_RING_A : (HAS_X ? FL_RING_X : FL_RING_N);
   static constexpr int K = K_, d = d_, D = K_ * d_;
   static constexpr int LPE = 8;                       // lanes per entry (factors padded to 8)
   static constexpr int EPS = 32 / LPE;                // entries per step
@@ -65,16 +77,25 @@ struct FlCfg {
   static constexpr int C4 = d_ / 4;                   // float4 chunks per factor slice
   static constexpr bool SHAPE_OK = (K_ <= LPE) && (d_ % 4 == 0) && (C4 == 1 || C4 == 2 || C4 == 4 || C4 == 8) &&
                                    (2 * K_ <= 32) && (K_ * C4 <= 64);
-  // d = 32: four 32-float slices per lane (own Z, own G, neighbour Z, accumulator) need ~170 registers
-  static constexpr int MAXW = (C4 == 8) ? (FL_MAXW < 12 ? FL_MAXW : 12) : FL_MAXW;
+  // d = 32: four 32-float slices per lane (own Z, own G, neighbour Z, accumulator) need ~170 registers;
+  // KEEPA holds three (own G, neighbour Z, accumulator).  KEEPA at d = 16 fits 128 registers (16 warps)
+  // without spilling; at 20 warps (96 registers) ptxas keeps loop-invariant values in local memory and
+  // reloads them every step, which measured 2.2x slower at mid (DESIGN 4.2)
+  static constexpr int MAXW_X = (C4 == 8) ? (FL_MAXW < 12 ? FL_MAXW : 12) : FL_MAXW;
+  static constexpr int MAXW_A = (C4 == 8) ? (FL_MAXW_A < 12 ? FL_MAXW_A : 12) : FL_MAXW_A;
+  static constexpr int MAXW = KEEPA ? MAXW_A : MAXW_X;
   static constexpr int ROWB = D * 4;
   static constexpr int ROWS = ((ROWB + 127) / 128) * 128;    // staged row stride (128-byte aligned)
   static constexpr int SLB = 128;                             // routed slice slot (d*4 <= 64 used)
   static constexpr int SRB = 128;                             // s[i,:], r[i,:] slot
-  static constexpr int OWN_B = 2 * ROWS + SRB;
+  // own-row slot: [Z[i]] G[i] (s, r)[i]
+  static constexpr int OWN_G = KEEPA ? 0 : ROWS;
+  static constexpr int OWN_SR = OWN_G + ROWS;
+  static constexpr int OWN_B = OWN_SR + SRB;
   static constexpr int NB_OFF = 0;
   static constexpr int SL_OFF = EPS * ROWS;
-  static constexpr int OWN_OFF = SL_OFF + (HAS_X ? 0 : EPS * SLB);
+  static constexpr int A_OFF = SL_OFF + (HAS_X ? 0 : EPS * SLB);   // KEEPA: a of the step's entries, EPS x 32 bytes
+  static constexpr int OWN_OFF = A_OFF + (KEEPA ? EPS * 32 : 0);
   static constexpr int STAGE_B = OWN_OFF + FL_OWN * OWN_B;
   static constexpr int BUDGET = 226 * 1024;
   static constexpr int NW_RAW = BUDGET / (FL_RING * STAGE_B);
@@ -192,7 +213,8 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
     const int rank = __popc(m.smask & sbits & (0xffffffffu >> (31 - lane))) - 1;
     m.info = (ks << 3) | (need ? 4 : 0) | (rank & 3);
   };
-  auto issue_stage = [&](unsigned st, const FMeta& m, int q) {
+  // cm = the chunk m describes (KEEPA: locates the entries' a)
+  auto issue_stage = [&](unsigned st, const FMeta& m, long long cm, int q) {
     const unsigned vq = (m.vmask >> (q * EPS)) & ((1u << EPS) - 1u);
     if (vq == 0) return;
 #pragma unroll
@@ -206,6 +228,10 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
       if (((vq >> grp) & 1u) && kap < C4)
         fl_cp16_small(st + C::SL_OFF + grp * C::SLB + kap * 16, G + cc * D + kk * d + kap * 4);
     }
+    if (C::KEEPA) {  // a[e, kap]: lane (e, kap) copies its own (EPS consecutive entries: 4 K contiguous floats)
+      if (((vq >> grp) & 1u) && factive)
+        fl_cp4(st + C::A_OFF + grp * 32 + kap * 4, coef_out + (cm * DL_CH + q * EPS + grp) * K + kap);
+    }
     if ((m.nmask >> (q * EPS)) & ((1u << EPS) - 1u)) {
       unsigned starts = (m.smask >> (q * EPS)) & ((1u << EPS) - 1u);
       int o = 0;
@@ -214,10 +240,10 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
         starts &= starts - 1;
         const long long node = g.row_base + __shfl_sync(DL_FULL, m.row, q * EPS + pos);
         const unsigned ow = st + C::OWN_OFF + o * OWN_B;
-        stage_row(ow, Z + node * D);
-        stage_row(ow + ROWS, G + node * D);
-        if (lane < K) fl_cp4(ow + 2 * ROWS + lane * 4, s + node * K + lane);
-        else if (lane < 2 * K) fl_cp4(ow + 2 * ROWS + lane * 4, r + node * K + (lane - K));
+        if (!C::KEEPA) stage_row(ow, Z + node * D);
+        stage_row(ow + C::OWN_G, G + node * D);
+        if (lane < K) fl_cp4(ow + C::OWN_SR + lane * 4, s + node * K + lane);
+        else if (lane < 2 * K) fl_cp4(ow + C::OWN_SR + lane * 4, r + node * K + (lane - K));
         ++o;
       }
     }
@@ -279,7 +305,7 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
   finish_meta(mA, c, -1);
 #pragma unroll
   for (int pq = 0; pq < FL_RING - 1; ++pq) {
-    issue_stage(ring + pq * STAGE_B, mA, pq);
+    issue_stage(ring + pq * STAGE_B, mA, c, pq);
     dl_cp_async_commit();
   }
   int rslot = 0;
@@ -306,8 +332,8 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
       int islot = rslot + (FL_RING - 1);
       if (islot >= FL_RING) islot -= FL_RING;
       const unsigned ist = ring + islot * STAGE_B;
-      if (q < QPC - (FL_RING - 1)) issue_stage(ist, mA, q + (FL_RING - 1));
-      else issue_stage(ist, mB, q + (FL_RING - 1) - QPC);
+      if (q < QPC - (FL_RING - 1)) issue_stage(ist, mA, c, q + (FL_RING - 1));
+      else issue_stage(ist, mB, cn, q + (FL_RING - 1) - QPC);
       dl_cp_async_commit();
       dl_cp_async_wait<FL_RING - 1>();
       __syncwarp();
@@ -328,16 +354,16 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
             const unsigned ow = st + C::OWN_OFF + rk * OWN_B;
 #pragma unroll
             for (int cc = 0; cc < C4; ++cc) {
-              zi[cc] = fl_lds4((ow + myblk) ^ (cc << 4));
-              gi[cc] = fl_lds4((ow + ROWS + myblk) ^ (cc << 4));
+              if (!C::KEEPA) zi[cc] = fl_lds4((ow + myblk) ^ (cc << 4));
+              gi[cc] = fl_lds4((ow + C::OWN_G + myblk) ^ (cc << 4));
             }
-            s_own = fl_lds1(ow + 2 * ROWS + kap * 4);
-            r_own = fl_lds1(ow + 2 * ROWS + (K + kap) * 4);
+            s_own = fl_lds1(ow + C::OWN_SR + kap * 4);
+            r_own = fl_lds1(ow + C::OWN_SR + (K + kap) * 4);
           } else {
             const long long node = g.row_base + row_e;
 #pragma unroll
             for (int cc = 0; cc < C4; ++cc) {
-              zi[cc] = dl_ldg4(Z + node * D + kap * d + cc * 4);
+              if (!C::KEEPA) zi[cc] = dl_ldg4(Z + node * D + kap * d + cc * 4);
               gi[cc] = dl_ldg4(G + node * D + kap * d + cc * 4);
             }
             s_own = __ldg(s + node * K + kap);
@@ -350,18 +376,25 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
           // (groups without a valid entry and idle factor lanes read stale bytes; they never reach dz)
           zj[cc] = fl_lds4((st + C::NB_OFF + grp * ROWS + myblk) ^ (cc << 4));
         }
-        float qv = fl_dot<C>(zi, zj);
-        if (!unit_T) qv = __fdiv_rn(qv, T);
-        const float ev = factive ? dl_expf(qv) : 0.0f;
-        // softmax denominator: the backward only needs a[] to ~1 ulp (kstar is read back, not
-        // recomputed), so the 8-lane butterfly and approximate reciprocals replace the forward's
+        // wv = a[kstar] and a[kap]: KEEPA reads the forward's (IEEE division by the sequential sum) back;
+        // otherwise they are recomputed, where the backward only needs a[] to ~1 ulp (kstar is read back,
+        // not recomputed), so the 8-lane butterfly and an approximate reciprocal replace the forward's
         // sequential sum and IEEE divisions
-        float sum = ev;
+        float wv, ev, rsum = 1.0f;                 // a[kap] = ev * rsum (KEEPA: ev = a[kap])
+        if (C::KEEPA) {
+          ev = fl_lds1(st + C::A_OFF + grp * 32 + kap * 4);
+          wv = __shfl_sync(DL_FULL, ev, gbase + ks);
+        } else {
+          float qv = fl_dot<C>(zi, zj);
+          if (!unit_T) qv = __fdiv_rn(qv, T);
+          ev = factive ? dl_expf(qv) : 0.0f;
+          float sum = ev;
 #pragma unroll
-        for (int off = 1; off < LPE; off <<= 1) sum = __fadd_rn(sum, __shfl_xor_sync(DL_FULL, sum, off));
-        const float eks = __shfl_sync(DL_FULL, ev, gbase + ks);
-        const float rsum = fl_rcp(sum);
-        const float wv = __fmul_rn(eks, rsum);
+          for (int off = 1; off < LPE; off <<= 1) sum = __fadd_rn(sum, __shfl_xor_sync(DL_FULL, sum, off));
+          const float eks = __shfl_sync(DL_FULL, ev, gbase + ks);
+          rsum = fl_rcp(sum);
+          wv = __fmul_rn(eks, rsum);
+        }
         const float cij = __fmul_rn(omb, __shfl_sync(DL_FULL, fl_dot<C>(gi, zj), gbase + ks));
         float cji;
         if (HAS_X) {
@@ -380,11 +413,12 @@ k_bwd_edges_fl(DlGraphDev g, const float* __restrict__ Z, const float* __restric
         float basec = __fmul_rn(dws, wv);
         if (!unit_T) basec = __fdiv_rn(basec, T);
         const float ind = (kap == ks) ? 1.0f : 0.0f;
-        float coef = __fmul_rn(basec, __fsub_rn(ind, __fmul_rn(ev, rsum)));
+        float coef = __fmul_rn(basec, __fsub_rn(ind, C::KEEPA ? ev : __fmul_rn(ev, rsum)));
         coef = (valid && factive) ? coef : 0.0f;
         // the coefficients are symmetric in (i, j): the lower-triangle phase reads them back instead of
-        // recomputing dots, exponentials and the softmax (32 contiguous bytes per entry at K = 8)
-        if (MODE == 2 && valid && factive) coef_out[(c * DL_CH + src) * K + kap] = coef;
+        // recomputing dots, exponentials and the softmax (32 contiguous bytes per entry at K = 8).  KEEPA:
+        // the same element held a[e, kap], staged above, so this overwrites what this lane already read.
+        if (MODE >= 2 && valid && factive) coef_out[(c * DL_CH + src) * K + kap] = coef;
         // accumulate: the whole step continues the current row (common), or run by run (entries of
         // a step are consecutive CSR entries)
         unsigned runs = (mA.smask >> (q * EPS)) & ((1u << EPS) - 1u);
@@ -499,15 +533,17 @@ int dl_launch_bwd_edges_fl(const DlGraphDev& g, const float* Z, const float* G, 
 
 // Symmetric pass 2, phase A: the kernel above on the upper-triangle view gu (entries with col >= row), kstar
 // and x in upper-view order (ku, xu); leaves the K coefficients of every upper entry in coef_out [nnz_u, K].
+// keep_a: coef_out holds the forward's softmax a [nnz_u, K] of the same entries (MODE 3), else it is recomputed.
 // (s, r) must already be packed in sr.  Returns -1000 when (K, d) has no instantiation.
 int dl_launch_bwd_sym_upper(const DlGraphDev& gu, const float* Z, const float* G, const unsigned char* ku,
                             const float* s, const float* r, const float2* sr, const float* xu, int K, int d, float omb,
-                            float T, float* dZ, float* coef_out, float* scratch, cudaStream_t st) {
+                            float T, float* dZ, float* coef_out, bool keep_a, float* scratch, cudaStream_t st) {
   if (!gu.erow || gu.nnz == 0 || !scratch || !dl_bwd_edges_fl_has(K, d) || !sr || !xu || !ku || !coef_out) return -1000;
   int rc = -1000;
-#define FL_CASE(KK, DD) \
-  if (K == KK && d == DD) \
-    rc = FlLaunch<KK, DD, 2>::run(gu, Z, G, ku, s, r, nullptr, sr, xu, omb, T, dZ, scratch, st, coef_out);
+#define FL_CASE(KK, DD)                                                                                   \
+  if (K == KK && d == DD)                                                                                 \
+    rc = keep_a ? FlLaunch<KK, DD, 3>::run(gu, Z, G, ku, s, r, nullptr, sr, xu, omb, T, dZ, scratch, st, coef_out) \
+                : FlLaunch<KK, DD, 2>::run(gu, Z, G, ku, s, r, nullptr, sr, xu, omb, T, dZ, scratch, st, coef_out);
   FL_CASE(8, 16)
   FL_CASE(8, 8)
   FL_CASE(5, 16)

@@ -8,7 +8,10 @@
 // (s, r) gathers only have to be done for ONE of the two entries.
 //
 //   phase A  k_bwd_edges_fl<K, d, 2> (bwd_fl.cu) on the upper-triangle view (col >= row): the full
-//            evaluation; adds coef * Z[j] to dZ[i] and stores coef [nnz_u, K] (coalesced, 4K bytes per entry)
+//            evaluation; adds coef * Z[j] to dZ[i] and stores coef [nnz_u, K] (coalesced, 4K bytes per entry).
+//            When the symmetric attention left its softmax a [nnz_u, K] in the same buffer (a_valid),
+//            k_bwd_edges_fl<K, d, 3> reads a there instead of recomputing the dots, exponentials and softmax,
+//            and overwrites it with coef
 //   phase B  k_bwd_sym_lower (here) on the strictly-lower view: gathers the row Z[j] and the mirror's K
 //            coefficients (one random 4K-byte access) and adds coef * Z[j] to dZ[i] -- ~1/4 of phase A's
 //            instructions per entry, no own-row state at all
@@ -250,7 +253,7 @@ int launch_lower(const DlGraphDev& g, const int* lmirror, const float* Z, const 
 bool dl_bwd_edges_fl_has(int K, int d);
 int dl_launch_bwd_sym_upper(const DlGraphDev& gu, const float* Z, const float* G, const unsigned char* ku,
                             const float* s, const float* r, const float2* sr, const float* xu, int K, int d, float omb,
-                            float T, float* dZ, float* coef_out, float* scratch, cudaStream_t st);
+                            float T, float* dZ, float* coef_out, bool keep_a, float* scratch, cudaStream_t st);
 void dl_pack_sr(const float* s, const float* r, long long n, float* sr_scratch, cudaStream_t st);
 
 extern "C" int dl_factor_bwd_edges_sym_supported(int K, int d) { return dl_bwd_edges_fl_has(K, d) ? 1 : 0; }
@@ -258,8 +261,8 @@ extern "C" int dl_factor_bwd_edges_sym_supported(int K, int d) { return dl_bwd_e
 extern "C" int dl_factor_bwd_edges_sym(const dl_graph* upper_host, const dl_graph* lower_host, const int32_t* lmirror,
                                        const float* Z, const float* G, const uint8_t* ku, const float* s, const float* r,
                                        float* sr_scratch, int64_t n_nodes, const float* xu, float* coef_scratch, int K,
-                                       int d, float one_minus_beta, float T, float* dZ, float* hub_ws,
-                                       dl_stream_t stream) {
+                                       int d, float one_minus_beta, float T, int a_valid, float* dZ,
+                                       float* hub_ws, dl_stream_t stream) {
   if (!dl_graph_ok(upper_host) || !dl_graph_ok(lower_host) || !dl_shape_ok(K, d)) return DL_EINVAL;
   if (upper_host->N != lower_host->N || upper_host->row_base != 0 || lower_host->row_base != 0) return DL_EINVAL;
   if (upper_host->N == 0 || upper_host->nnz == 0) return DL_OK;
@@ -273,9 +276,10 @@ extern "C" int dl_factor_bwd_edges_sym(const dl_graph* upper_host, const dl_grap
   const DlGraphDev gl = dl_graph_dev(lower_host);
   dl_pack_sr(s, r, (long long)n_nodes * K, sr_scratch, st);
   DL_LAUNCH_CHECK();
+  const bool keep_a = a_valid && !(upper_host->flags & DL_F_NO_KEEPA);
   int rc = dl_launch_bwd_sym_upper(gu, Z, G, ku, s, r,
                                    reinterpret_cast<const float2*>(sr_scratch), xu, K, d, one_minus_beta, T, dZ,
-                                   coef_scratch, hub_ws, st);
+                                   coef_scratch, keep_a, hub_ws, st);
   if (rc == -1000) return DL_EUNSUPPORTED;
   if (rc) return rc;
   if (gl.nnz == 0) return DL_OK;

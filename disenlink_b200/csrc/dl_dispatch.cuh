@@ -135,5 +135,6 @@ int dl_launch_bwd_edges_fl(const DlGraphDev& g, const float* Z, const float* G, 
 // Factor-per-lane attention + row sums (attn_fl.cu).  Returns -1000 when (K, d) has no instantiation.
 int dl_gather_chain_rowsum(const DlGraphDev& g, int K, float* scratch, float* s_out, cudaStream_t st);
 int dl_launch_attn_fl(const DlGraphDev& g, const float* Z, int K, int d, float T, unsigned char* kstar,
-                      float* w, float* s, float* scratch, cudaStream_t st, float2* kw_out = nullptr);
+                      float* w, float* s, float* scratch, cudaStream_t st, float2* kw_out = nullptr,
+                      float* a_out = nullptr);
 bool dl_attn_fl_has(int K, int d);

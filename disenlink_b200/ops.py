@@ -38,9 +38,11 @@ def _check_Z(Z: torch.Tensor, n_nodes: int):
 # --------------------------------------------------------------------------------------------
 # raw kernel wrappers (no autograd)
 # --------------------------------------------------------------------------------------------
-def edge_attn_fwd(graph: Graph, Z: torch.Tensor, T: float = 1.0, out=None):
+def edge_attn_fwd(graph: Graph, Z: torch.Tensor, T: float = 1.0, out=None, plan: dict = None):
     """-> (kstar u8 [nnz], w f32 [nnz], s f32 [N,K]).  [ref: model.py:56-73]
-    `out` = optional preallocated (kstar, w, s)."""
+    `out` = optional preallocated (kstar, w, s).  `plan` = the bwd_plan of the backward that follows with the
+    same Z and T: in mode "sym" the symmetric attention leaves its softmax in plan["coef"] and sets
+    plan["a_valid"], and backward pass 2 reads it instead of recomputing it (off under DL_F_NO_KEEPA)."""
     K, d = _check_Z(Z, graph.n_global)
     Z = Z.contiguous()
     dev = Z.device
@@ -53,6 +55,11 @@ def edge_attn_fwd(graph: Graph, Z: torch.Tensor, T: float = 1.0, out=None):
             s = torch.empty(graph.n_global, K, dtype=torch.float32, device=dev)
         rc = _lib.DL_EUNSUPPORTED
         sym = None
+        a_out = None
+        if plan is not None:
+            plan["a_valid"] = False
+            if plan["mode"] == "sym" and not (graph.flags & _lib.DL_F_NO_KEEPA):
+                a_out = plan["coef"]
         if graph.nnz >= graph.sym_min_nnz and not (graph.flags & (_lib.DL_F_NO_SYM | _lib.DL_F_NO_STREAM |
                                                                   _lib.DL_F_NO_FL | _lib.DL_F_NO_FL_ATTN)):
             sym = graph.sym_view()              # None: not symmetric / row-partitioned
@@ -61,9 +68,12 @@ def edge_attn_fwd(graph: Graph, Z: torch.Tensor, T: float = 1.0, out=None):
             upper, eidx = sym
             kw = _x_scratch(graph, 2 * upper.nnz)
             rc = lib().dl_edge_attn_fwd_sym(graph.ref, upper.ref, ptr(eidx), ptr(Z), K, d, float(T), ptr(kstar),
-                                            ptr(w), ptr(s), ptr(graph.hub_scratch(K)), ptr(kw), stream_of(dev))
+                                            ptr(w), ptr(s), ptr(graph.hub_scratch(K)), ptr(kw), _optr(a_out),
+                                            stream_of(dev))
             if rc != _lib.DL_EUNSUPPORTED:
                 check(rc, "dl_edge_attn_fwd_sym")
+                if a_out is not None:
+                    plan["a_valid"] = True
         if rc == _lib.DL_EUNSUPPORTED:
             check(lib().dl_edge_attn_fwd(graph.ref, ptr(Z), K, d, float(T), ptr(kstar), ptr(w), ptr(s),
                                          ptr(graph.hub_scratch(K)), stream_of(dev)), "dl_edge_attn_fwd")
@@ -114,8 +124,10 @@ def bwd_plan(graph: Graph, K: int, d: int, allow_sym: bool = True) -> dict:
                    transient scratch -- when that does not fit, mode "x" is used
       mode "x"     pass 1 leaves the per-entry dots for every entry, pass 2 reads them (dl_factor_bwd_edges)
     The per-entry scratch is the graph's cached one (shared with the symmetric attention's packed records,
-    which are dead by the time the backward runs)."""
-    plan = {"mode": "x", "x": _x_scratch(graph), "x_valid": False}
+    which are dead by the time the backward runs).  In mode "sym", a forward given the plan (edge_attn_fwd)
+    stores the softmax of the upper entries in "coef" and sets "a_valid"; pass 2 then reads it and clears
+    "a_valid", since the buffer holds coefficients afterwards."""
+    plan = {"mode": "x", "x": _x_scratch(graph), "x_valid": False, "a_valid": False}
     f = graph.flags
     if (allow_sym and graph.nnz >= graph.sym_min_nnz and graph.nnz > 0 and
             not (f & (_lib.DL_F_NO_SYM | _lib.DL_F_NO_STREAM | _lib.DL_F_NO_FL | _lib.DL_F_NO_XDOT)) and
@@ -189,11 +201,13 @@ def factor_bwd_edges(graph: Graph, Z, G, kstar, w, s, r, beta: float, T: float, 
     valid = plan is not None and plan.get("x_valid")
     with torch.cuda.device(dev):
         if valid and plan["mode"] == "sym":
+            a_valid = 1 if plan.get("a_valid") else 0
+            plan["a_valid"] = False                        # from here on coef holds coefficients
             check(lib().dl_factor_bwd_edges_sym(plan["upper"].ref, plan["lower"].ref, ptr(plan["lmirror"]), ptr(Z), ptr(G),
                                                 ptr(plan["ku"]), ptr(s), ptr(r), ptr(_sr_scratch(graph, s)),
                                                 int(s.shape[0]), ptr(plan["xu"]), ptr(plan["coef"]), K, d,
-                                                one_minus(beta), float(T), ptr(dZ), ptr(graph.hub_scratch(K * d)),
-                                                stream_of(dev)), "dl_factor_bwd_edges_sym")
+                                                one_minus(beta), float(T), a_valid, ptr(dZ),
+                                                ptr(graph.hub_scratch(K * d)), stream_of(dev)), "dl_factor_bwd_edges_sym")
             return
         if plan is not None and plan["mode"] == "sym":
             raise RuntimeError("pass 1 did not fill the upper-view dots the symmetric pass 2 was planned on")

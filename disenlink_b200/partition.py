@@ -507,8 +507,8 @@ class CudaBackend:
                   "dl_need_masks")
 
     # -- kernels (all write only the owned rows [0, n_own) of the local arrays) --
-    def edge_attn_fwd(self, g, Z, T, kstar, w, s):
-        self.ops.edge_attn_fwd(g, Z, T, out=(kstar, w, s))
+    def edge_attn_fwd(self, g, Z, T, kstar, w, s, plan=None):
+        self.ops.edge_attn_fwd(g, Z, T, out=(kstar, w, s), plan=plan)
 
     def factor_spmm_fwd(self, g, Z, kstar, w, s, beta, H, sj=None, zs=None):
         self.ops.factor_spmm_fwd(g, Z, kstar, w, s, beta, out=H, sj=sj, zs=zs)
@@ -657,7 +657,11 @@ class PartitionedLinkStep:
         mark("wait")                 # what the slowest rank of the previous step costs everybody (load imbalance)
         px.push_rows(Z, plan.send_all, plan.recv_all, dst_base=plan.dst_base)
         mark("ag_Z")
-        be.edge_attn_fwd(g, Z, self.T, self.kstar, self.w, self.s)
+        if self.plan_bwd is not None:
+            # the symmetric attention leaves its softmax in the plan's coefficient buffer for backward pass 2
+            be.edge_attn_fwd(g, Z, self.T, self.kstar, self.w, self.s, plan=self.plan_bwd)
+        else:
+            be.edge_attn_fwd(g, Z, self.T, self.kstar, self.w, self.s)
         mark("attn_fwd")
         if part.world > 1:
             if hasattr(be, "need_masks"):

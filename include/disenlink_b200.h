@@ -135,6 +135,8 @@ typedef struct dl_graph {
                                  per-entry dot pass 1 left in x */
 #define DL_F_NO_SYM 128u      /* (host side) attention evaluates both directions of every edge even when
                                  the symmetric path (dl_edge_attn_fwd_sym) is available */
+#define DL_F_NO_KEEPA 256u    /* the symmetric attention does not store its softmax (a_out is ignored) and the
+                                 symmetric backward pass 2 recomputes it (a_valid is ignored) */
 
 /* ------------------------------------------------------------------------------------------
  * (2) per-edge K-factor attention with hard routing.
@@ -168,14 +170,18 @@ int dl_edge_attn_fwd(const dl_graph* g_host, const float* Z, int K, int d, float
  *       a streaming pass expands them through eidx into kstar / w of the full CSR and makes the row
  *       sums s.  Outputs are identical to dl_edge_attn_fwd (kstar, w bit for bit; s up to the order of
  *       the fp32 row sums).  hub_ws: dl_hub_scratch_floats(g, K) floats.  DL_EUNSUPPORTED when (K, d) has
- *       no factor-per-lane instantiation: call dl_edge_attn_fwd instead.  [ref: model.py:56-73] */
+ *       no factor-per-lane instantiation: call dl_edge_attn_fwd instead.
+ *       a_out (may be NULL; ignored under DL_F_NO_KEEPA in g_host->flags): nnz_u K floats that receive the
+ *       softmax a[t, k] of every primary entry t (the bits w is taken from).  Handed to
+ *       dl_factor_bwd_edges_sym as its coef_scratch with a_valid = 1, it spares backward pass 2 the dots,
+ *       exponentials and softmax.  [ref: model.py:56-73] */
 size_t dl_sym_index_workspace_bytes(int64_t N, int64_t nnz);
 int dl_sym_index(const int64_t* rowptr, const int32_t* col, const int32_t* erow, int64_t N, int64_t nnz,
                  int64_t* uptr, int32_t* ucol, int32_t* eidx, int32_t* lcol, int32_t* lmirror, int32_t* status_out,
                  void* ws, size_t ws_bytes, dl_stream_t stream);
 int dl_edge_attn_fwd_sym(const dl_graph* g_host, const dl_graph* upper_host, const int32_t* eidx, const float* Z,
                          int K, int d, float T, uint8_t* kstar, float* w, float* s, float* hub_ws,
-                         float* kw_scratch, dl_stream_t stream);
+                         float* kw_scratch, float* a_out, dl_stream_t stream);
 
 /* (3) per-factor gather / segment-sum aggregation with the beta residual.
  * [ref: model.py:75]  H[i,k] = beta Z[i,k] + (1-beta) sum_{j: kstar(i,j)=k} w_ij / s[j,k] Z[j,k]
@@ -227,12 +233,16 @@ int dl_factor_bwd_gather(const dl_graph* g_host, const float* Z, const float* G,
  * <G[j,k*], Z[i,k*]> in upper-view order (dl_factor_bwd_gather with x_index); sr_scratch: 2 n_nodes K floats;
  * coef_scratch: nnz_u K floats; hub_ws: dl_hub_scratch_floats(full graph, K*d) floats.  dZ is accumulated
  * into.  Equal to dl_factor_bwd_edges up to fp32 rounding (the two directions of an edge associate dwsum and
- * the row sums differently).  DL_EUNSUPPORTED when (K, d) has no factor-per-lane instantiation. */
+ * the row sums differently).  DL_EUNSUPPORTED when (K, d) has no factor-per-lane instantiation.
+ * a_valid != 0: coef_scratch holds the softmax dl_edge_attn_fwd_sym stored through a_out for the same Z, T
+ * and views; phase A reads it instead of recomputing it (and without the rows Z[i]), and overwrites it with
+ * the coefficients, so the caller clears its record of a valid softmax after this call.  Ignored under
+ * DL_F_NO_KEEPA in upper_host->flags. */
 int dl_factor_bwd_edges_sym_supported(int K, int d);     /* 1 when (K, d) has the kernels, else 0 */
 int dl_factor_bwd_edges_sym(const dl_graph* upper_host, const dl_graph* lower_host, const int32_t* lmirror,
                             const float* Z, const float* G, const uint8_t* ku, const float* s, const float* r,
                             float* sr_scratch, int64_t n_nodes, const float* xu, float* coef_scratch, int K, int d,
-                            float one_minus_beta, float T, float* dZ, float* hub_ws, dl_stream_t stream);
+                            float one_minus_beta, float T, int a_valid, float* dZ, float* hub_ws, dl_stream_t stream);
 int dl_factor_bwd_edges(const dl_graph* g_host, const float* Z, const float* G,
                         const uint8_t* kstar, const float* w, const float* s, const float* r,
                         const float* sj, float* sr_scratch, int64_t n_nodes, const float* x, int K,
