@@ -72,6 +72,8 @@ SIGNATURES = {
     "dl_csr_from_dense": (_int, [_vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "dl_entry_rows": (_int, [_vp, _i64, _i64, _vp, _vp]),
     "dl_rev_index": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp]),
+    "dl_transpose_index_workspace_bytes": (_sz, [_i64, _i64]),
+    "dl_transpose_index": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
     "dl_degree_buckets_workspace_bytes": (_sz, [_i64]),
     "dl_degree_buckets": (_int, [_vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "dl_hub_items": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _vp]),
@@ -87,6 +89,8 @@ SIGNATURES = {
     "dl_factor_bwd_edges_sym": (_int, [_GP, _GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _int, _int, _f, _f, _int,
                                        _vp, _vp, _vp]),
     "dl_factor_bwd_edges": (_int, [_GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _int, _int, _f, _f, _vp, _vp, _vp]),
+    "dl_factor_bwd_directed": (_int, [_GP, _GP, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _f, _f, _f, _vp, _vp, _vp, _vp,
+                                      _vp, _vp, _vp]),
     "dl_pair_score_fwd": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _int, _int, _f, _vp, _vp, _vp]),
     "dl_pair_incidence_workspace_bytes": (_sz, [_i64, _i64]),
     "dl_pair_incidence": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ_DIR = os.path.join(HERE, "_obj")
 LIB = os.path.join(HERE, "libdisenlink_b200.so")
 VARIANT_DIR = os.path.join(HERE, "_variants")
-SOURCES = ["graph_build.cu", "factor_fwd.cu", "attn_stream.cu", "attn_fl.cu", "attn_sym.cu", "gather_stream.cu", "bwd_stream.cu", "bwd_fl.cu", "bwd_sym.cu", "slice_gather.cu", "factor_bwd.cu",
+SOURCES = ["graph_build.cu", "factor_fwd.cu", "attn_stream.cu", "attn_fl.cu", "attn_sym.cu", "gather_stream.cu", "bwd_stream.cu", "bwd_fl.cu", "bwd_sym.cu", "slice_gather.cu", "factor_bwd.cu", "bwd_dir.cu",
            "pair_score.cu", "pair_stream.cu", "link_loss.cu", "eval_metrics.cu", "sampling.cu", "peer_copy.cu", "dense_compat.cu"]
 HEADERS = [os.path.join(CSRC, h) for h in ("dl_common.cuh", "dl_dispatch.cuh", "dl_stream.cuh", "dl_fl.cuh", "dl_prims.cuh")] + [
     os.path.join(os.path.dirname(HERE), "include", "disenlink_b200.h")]

@@ -1,5 +1,5 @@
 // graph_build.cu -- integer work: adjacency -> CSR, reverse-edge index, degree buckets, hub work
-// items, pair incidence lists.  All outputs are bit-exact functions of the inputs (no float, no
+// items, pair incidence lists, transposed pattern.  All outputs are bit-exact functions of the inputs (no float, no
 // order-dependent atomics).
 //
 // Reference being replaced: main_disentangled.py:137-142 builds a dense [N,N] adj_sym from the
@@ -261,6 +261,31 @@ __global__ void k_incidence_decode(const unsigned* __restrict__ skey, const unsi
   }
 }
 
+// ---- transposed pattern -----------------------------------------------------------------------
+// key = column (the node the entry points to), value = CSR entry index; the stable sort keeps the
+// in-entries of a node in CSR order (ascending source row)
+__global__ void k_transpose_keys(const int* __restrict__ col, long long nnz, unsigned* __restrict__ key,
+                                 unsigned* __restrict__ val) {
+  long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += stride) {
+    key[e] = (unsigned)col[e];
+    val[e] = (unsigned)e;
+  }
+}
+
+__global__ void k_transpose_decode(const unsigned* __restrict__ skey, const unsigned* __restrict__ sval,
+                                   const int* __restrict__ erow, long long nnz, long long N, int* __restrict__ tcol,
+                                   int* __restrict__ tperm, long long* __restrict__ marks) {
+  long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < nnz; t += stride) {
+    const unsigned e = sval[t];
+    tperm[t] = (int)e;
+    tcol[t] = erow[e];
+    const unsigned node = skey[t];
+    if (node < N && (t + 1 == nnz || skey[t + 1] != node)) marks[(long long)node + 1] = t + 1;
+  }
+}
+
 inline int blocks_for(long long n, int threads = 256, int cap = 148 * 32) {
   long long b = (n + threads - 1) / threads;
   if (b < 1) b = 1;
@@ -473,6 +498,45 @@ int dl_pair_incidence_range(const int32_t* u, const int32_t* v, int64_t P, int64
   (void)cub_bytes;
   return dlp::scan<true, long long>(dlp::LoadArr<long long>{marks}, dlp::StoreArr<long long>{(long long*)inc_ptr}, N + 1,
                                     dlp::OpMax<long long>(), 0LL, cub_ws, st);
+}
+
+static size_t transpose_sort_bytes(long long nnz, long long N) {
+  const size_t a = dlp::sort_ws_bytes(nnz > 0 ? nnz : 1), c = dlp::scan_ws_bytes(N + 1, 8);
+  return a > c ? a : c;
+}
+
+size_t dl_transpose_index_workspace_bytes(int64_t N, int64_t nnz) {
+  if (N < 0 || nnz < 0) return 0;
+  size_t m = (size_t)(nnz > 0 ? nnz : 1);
+  return 4 * align256(m * 4) + align256((size_t)(N + 1) * 8) + align256(transpose_sort_bytes(nnz, N));
+}
+
+int dl_transpose_index(const int32_t* col, const int32_t* erow, int64_t N, int64_t nnz, int64_t* trowptr,
+                       int32_t* tcol, int32_t* tperm, void* ws, size_t ws_bytes, dl_stream_t stream) {
+  if (N < 0 || N >= (1LL << 31) - 1 || nnz < 0 || nnz >= (1LL << 31) - 1) return DL_EINVAL;
+  if (!trowptr || !ws || (nnz > 0 && (!col || !erow || !tcol || !tperm))) return DL_EINVAL;
+  if (ws_bytes < dl_transpose_index_workspace_bytes(N, nnz)) return DL_EWORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  size_t m = (size_t)(nnz > 0 ? nnz : 1);
+  char* base = (char*)ws;
+  unsigned* key_in = (unsigned*)base;
+  unsigned* key_out = (unsigned*)(base + align256(m * 4));
+  unsigned* val_in = (unsigned*)(base + 2 * align256(m * 4));
+  unsigned* val_out = (unsigned*)(base + 3 * align256(m * 4));
+  long long* marks = (long long*)(base + 4 * align256(m * 4));
+  void* sort_ws = base + 4 * align256(m * 4) + align256((size_t)(N + 1) * 8);
+  DL_CUDA_TRY(cudaMemsetAsync(marks, 0, (size_t)(N + 1) * 8, st));
+  if (nnz > 0) {
+    k_transpose_keys<<<blocks_for(nnz), 256, 0, st>>>(col, nnz, key_in, val_in);
+    DL_LAUNCH_CHECK();
+    const int bits = dl_bits_for(N > 1 ? N : 2);
+    int rc = dlp::sort_pairs<unsigned, unsigned>(key_in, key_out, val_in, val_out, nnz, 0, bits, sort_ws, st);
+    if (rc) return rc;
+    k_transpose_decode<<<blocks_for(nnz), 256, 0, st>>>(key_out, val_out, erow, nnz, N, tcol, tperm, marks);
+    DL_LAUNCH_CHECK();
+  }
+  return dlp::scan<true, long long>(dlp::LoadArr<long long>{marks}, dlp::StoreArr<long long>{(long long*)trowptr},
+                                    N + 1, dlp::OpMax<long long>(), 0LL, sort_ws, st);
 }
 
 }  // extern "C"

@@ -25,6 +25,10 @@ class Graph:
     ``adj_sym.nonzero()``.  ``perm`` lists rows by degree class (bit length of the degree)
     descending; rows with degree >= 512 are "hub rows" and are cut into 512-edge segments so no
     warp owns more than one segment.
+
+    ``directed`` marks a pattern that is used as given, not as an undirected graph: its backward runs
+    over the pattern and its transpose (transpose_view) and accepts any 0/1 adjacency, symmetric or not.
+    An unmarked graph needs a symmetric pattern for the backward (DL_EASYM otherwise).
     """
 
     # below this many entries the attention runs two-sided: the graph fits L2 and the extra launches
@@ -32,7 +36,7 @@ class Graph:
     SYM_MIN_NNZ = 1 << 20
 
     def __init__(self, rowptr: torch.Tensor, col: torch.Tensor, n_nodes: int, row_base: int = 0,
-                 n_global: int = None):
+                 n_global: int = None, directed: bool = False):
         require_cuda(rowptr, "rowptr")
         assert rowptr.dtype == torch.int64 and col.dtype == torch.int32
         self.device = rowptr.device
@@ -45,16 +49,20 @@ class Graph:
         self._rev = None
         self._sym = None                      # (upper Graph, eidx) | False (pattern not symmetric / unavailable)
         self._sym_lower = None
+        self._transpose = None                # (transposed Graph, tperm int32 [nnz])
+        self.directed = bool(directed)
         self.sym_min_nnz = self.SYM_MIN_NNZ
         self._flags = _lib.default_flags()
         self._build_items()
 
     # ------------------------------------------------------------------ constructors
     @classmethod
-    def from_edges(cls, src: torch.Tensor, dst: torch.Tensor, n_nodes: int, symmetrize: bool = True) -> "Graph":
+    def from_edges(cls, src: torch.Tensor, dst: torch.Tensor, n_nodes: int, symmetrize: bool = None,
+                   directed: bool = False) -> "Graph":
         """Symmetrise + de-duplicate directed edge columns (self-loops kept).
         ``symmetrize=False`` keeps the directed columns as they are (de-duplicated) -- the edge set
-        structured negative sampling tests membership against.
+        structured negative sampling tests membership against.  ``directed=True`` marks the graph
+        directed (see the class doc) and keeps the columns as given unless ``symmetrize=True``.
 
         [ref: main_disentangled.py:137-142]"""
         require_cuda(src, "src")
@@ -63,6 +71,8 @@ class Graph:
         dst = dst.to(torch.int64).contiguous()
         E = int(src.numel())
         N = int(n_nodes)
+        if symmetrize is None:
+            symmetrize = not directed
         L = lib()
         with torch.cuda.device(dev):
             rowptr = torch.empty(N + 1, dtype=torch.int64, device=dev)
@@ -84,14 +94,15 @@ class Graph:
                 raise _lib.DlError(status, "dl_csr_build")
             del ws
             col = col[:nnz].clone() if nnz < col.numel() else col
-        return cls(rowptr, col, N)
+        return cls(rowptr, col, N, directed=directed)
 
     @classmethod
-    def from_edge_index(cls, edge_index: torch.Tensor, n_nodes: int) -> "Graph":
-        return cls.from_edges(edge_index[0], edge_index[1], n_nodes)
+    def from_edge_index(cls, edge_index: torch.Tensor, n_nodes: int, directed: bool = False) -> "Graph":
+        """Symmetrised, or with ``directed=True`` the columns as given (de-duplicated), marked directed."""
+        return cls.from_edges(edge_index[0], edge_index[1], n_nodes, directed=directed)
 
     @classmethod
-    def from_dense(cls, adj: torch.Tensor) -> "Graph":
+    def from_dense(cls, adj: torch.Tensor, directed: bool = False) -> "Graph":
         """From the dense adjacency the reference passes to ``Disentangle.forward`` (used as is,
         any non-zero entry is an edge).  [ref: model.py:62]"""
         require_cuda(adj, "adj")
@@ -110,11 +121,11 @@ class Graph:
             col = torch.empty(max(nnz, 1), dtype=torch.int32, device=dev)
             check(L.dl_csr_from_dense(ptr(a), N, ptr(rowptr), ptr(col), None, 0, stream_of(dev)),
                   "dl_csr_from_dense(fill)")
-        return cls(rowptr, col[:nnz], N)
+        return cls(rowptr, col[:nnz], N, directed=directed)
 
     @classmethod
-    def from_csr(cls, rowptr: torch.Tensor, col: torch.Tensor) -> "Graph":
-        return cls(rowptr.to(torch.int64), col.to(torch.int32), int(rowptr.numel()) - 1)
+    def from_csr(cls, rowptr: torch.Tensor, col: torch.Tensor, directed: bool = False) -> "Graph":
+        return cls(rowptr.to(torch.int64), col.to(torch.int32), int(rowptr.numel()) - 1, directed=directed)
 
     # ------------------------------------------------------------------ integer kernels
     def _build_items(self) -> None:
@@ -248,6 +259,30 @@ class Graph:
         """-> (strictly-lower-triangle Graph, lmirror int32 [nnz_l] = upper-view position of every lower entry's
         mirror) for the symmetric backward pass 2, or None (see sym_view)."""
         return self._sym_lower if self.sym_view() is not None else None
+
+    def transpose_view(self):
+        """-> (transposed Graph, tperm int32 [nnz]): row j of the transposed graph lists the in-entries of
+        node j (their source rows, in CSR order) and tperm[p] is the CSR index of in-entry p.  A graph of its
+        own, so in-hubs get degree buckets and hub work items; the directed backward gathers over it.  Needs
+        row_base == 0 (one GPU) and nnz < 2^31 - 1.  Integer work on the device, done once and cached."""
+        if self._transpose is None:
+            if self.row_base != 0 or self.n_global != self.N or self.nnz >= 2**31 - 1:
+                raise ValueError("the transposed view needs a whole graph on one GPU (row_base 0, nnz < 2^31 - 1)")
+            L, dev, N = lib(), self.device, self.N
+            with torch.cuda.device(dev):
+                trowptr = torch.empty(N + 1, dtype=torch.int64, device=dev)
+                tcol = torch.empty(max(self.nnz, 1), dtype=torch.int32, device=dev)
+                tperm = torch.empty(max(self.nnz, 1), dtype=torch.int32, device=dev)
+                ws_bytes = L.dl_transpose_index_workspace_bytes(N, self.nnz)
+                ws = _ws(ws_bytes, dev)
+                check(L.dl_transpose_index(ptr(self.col), ptr(self.erow), N, self.nnz, ptr(trowptr), ptr(tcol),
+                                           ptr(tperm), ptr(ws), ws_bytes, stream_of(dev)), "dl_transpose_index")
+                del ws
+            tg = Graph(trowptr, tcol[:self.nnz], N)
+            tg._sym = False
+            tg.flags = self._flags
+            self._transpose = (tg, tperm[:self.nnz])
+        return self._transpose
 
     def rows(self) -> torch.Tensor:
         """Row id of every entry (torch op; for tests and dense views)."""

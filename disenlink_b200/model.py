@@ -146,39 +146,41 @@ class _GraphCache:
         self._version = None
         self._graph: Optional[Graph] = None
 
-    def get(self, adj: AdjLike, n_nodes: int) -> Graph:
+    def get(self, adj: AdjLike, n_nodes: int, directed: bool = False) -> Graph:
+        """A Graph is used as it is (marked or not); a tensor is turned into a graph marked ``directed``."""
         if isinstance(adj, Graph):
             return adj
         if not isinstance(adj, torch.Tensor):
             raise TypeError("adj must be a dense [N,N] tensor, an edge_index [2,E] tensor or a Graph")
         # keyed on the tensor OBJECT (a weak reference) and its version counter: an address is not an
         # identity -- the caching allocator hands a freed adjacency's address to the next one of that shape
-        same = self._ref is not None and self._ref() is adj and self._version == adj._version
+        same = (self._ref is not None and self._ref() is adj and self._version == adj._version
+                and self._graph.directed == bool(directed))
         if not same:
             require_cuda(adj, "adj")
             sparse = adj.layout != torch.strided        # checked before anything touches data_ptr()
             if sparse:
                 coo = (adj.to_sparse_coo() if adj.layout != torch.sparse_coo else adj).coalesce()
                 idx = coo.indices()[:, coo.values() != 0]
-                rp_graph = _graph_from_entries(idx[0], idx[1], n_nodes)
+                rp_graph = _graph_from_entries(idx[0], idx[1], n_nodes, directed)
             elif adj.dim() == 2 and adj.shape[0] == 2 and not adj.is_floating_point():
-                rp_graph = Graph.from_edge_index(adj, n_nodes)
+                rp_graph = Graph.from_edge_index(adj, n_nodes, directed=directed)
             elif adj.dim() == 2 and adj.shape[0] == adj.shape[1] == n_nodes:
-                rp_graph = Graph.from_dense(adj)
+                rp_graph = Graph.from_dense(adj, directed=directed)
             else:
                 raise ValueError(f"cannot interpret adj of shape {tuple(adj.shape)} for N={n_nodes}")
             self._ref, self._version, self._graph = weakref.ref(adj), adj._version, rp_graph
         return self._graph
 
 
-def _graph_from_entries(row, col, n_nodes):
+def _graph_from_entries(row, col, n_nodes, directed=False):
     """Entries used as given (no symmetrisation): sort + unique through the edge kernel would
     symmetrise, so build the CSR from sorted keys with torch integer ops (one-off, tiny)."""
     key = torch.unique(row.to(torch.int64) * n_nodes + col.to(torch.int64))
     r, c = key // n_nodes, (key % n_nodes).to(torch.int32)
     rowptr = torch.zeros(n_nodes + 1, dtype=torch.int64, device=row.device)
     rowptr[1:] = torch.cumsum(torch.bincount(r, minlength=n_nodes), 0)
-    return Graph(rowptr, c, n_nodes)
+    return Graph(rowptr, c, n_nodes, directed=directed)
 
 
 def is_dense_adj(adj: AdjLike, n_nodes: int) -> bool:
@@ -201,10 +203,19 @@ class Disentangle_layer(nn.Module):
         self.beta = beta
         self.dense_limit = dense_limit
         self._cache = _GraphCache()
+        # how a tensor adj is read: "symmetric" (an undirected graph like the script's adj_sym; the backward
+        # refuses a pattern that is not symmetric) or "directed" (any 0/1 pattern, used as given; the backward
+        # gathers over its transpose).  A Graph handle carries its own mark (Graph.directed).
+        self.adjacency = "symmetric"
+
+    def _directed(self) -> bool:
+        if self.adjacency not in ("symmetric", "directed"):
+            raise ValueError(f"adjacency must be 'symmetric' or 'directed', got {self.adjacency!r}")
+        return self.adjacency == "directed"
 
     def sparse_forward(self, Z: torch.Tensor, adj: AdjLike):
         """Z [N,K,d] -> (H [N,K,d], kstar u8 [nnz], w [nnz], s [N,K], graph)."""
-        graph = self._cache.get(adj, Z.shape[0])
+        graph = self._cache.get(adj, Z.shape[0], self._directed())
         H, kstar, w, s = ops.factor_aggregate(Z, graph, self.beta, float(self.temperature),
                                               return_attention=True)
         return H, kstar, w, s, graph
@@ -289,6 +300,19 @@ class Disentangle(nn.Module):
         # "fp32": plain SGEMM (default, bit-compatible with the reference's nn.Linear on the same library);
         # "3xtf32": three TF32 tensor-core GEMMs per product, fp32-class accuracy (dense CUDA x only)
         self.projection = "fp32"
+
+    @property
+    def adjacency(self) -> str:
+        """"symmetric" (default): a tensor adj is an undirected graph such as adj_sym, and the backward
+        refuses a pattern that is not symmetric.  "directed": a dense, sparse or edge_index adj is used as
+        given (edge_index columns are not symmetrised) and trains through the backward over its transpose,
+        e.g. the directed train adjacency.  A Graph handle passed as adj carries its own mark."""
+        return self.disentangle_layer1.adjacency
+
+    @adjacency.setter
+    def adjacency(self, value: str) -> None:
+        self.disentangle_layer1.adjacency = value
+        self.disentangle_layer2.adjacency = value
 
     def project(self, x: torch.Tensor) -> torch.Tensor:
         """Z [N,K,d] = the K factor MLPs of model.py:106, batched: one [N,F] x [F,K*nhid] GEMM for the

@@ -1,6 +1,7 @@
 """torch.autograd bindings of the hot-path kernels (C ABI in include/disenlink_b200.h).
 
-    factor_aggregate(Z, graph, beta, T)  -> H            model.py:56-75   (attention + aggregation)
+    factor_aggregate(Z, graph, beta, T)  -> H            model.py:56-75   (attention + aggregation; any
+                                                         pattern when the graph is marked directed)
     PairBatch(u, v, N) / pair_score(Z, H, batch, T)      model.py:109-113 on explicit pairs
     allpairs_score(Z, H, T)              -> [N,N]        model.py:109-113 dense (small-N drop-in)
 
@@ -239,6 +240,29 @@ def factor_bwd(graph: Graph, Z, G, kstar, w, s, beta: float, T: float = 1.0, dZ=
     return dZ, r
 
 
+def factor_bwd_directed(graph: Graph, Z, G, kstar, w, s, beta: float, T: float = 1.0, dZ=None, r=None):
+    """dL/dZ through attention + aggregation for ANY 0/1 pattern (graphs marked directed), given
+    G = dL/dH; accumulated into dZ if given.  Gathers over the pattern and its transpose
+    (Graph.transpose_view; csrc/bwd_dir.cu).  -> (dZ, r), r = 0 where a (node, factor) has no routed
+    out-entry.  [ref: autograd of model.py:56-75]"""
+    K, d = _check_Z(Z, graph.n_global)
+    Z = Z.contiguous()
+    G = G.contiguous()
+    dev = Z.device
+    tg, tperm = graph.transpose_view()
+    with torch.cuda.device(dev):
+        if dZ is None:
+            dZ = torch.zeros_like(Z)
+        if r is None:
+            r = torch.empty(graph.N, K, dtype=torch.float32, device=dev)
+        routed = torch.empty(max(graph.N, 1), dtype=torch.int32, device=dev)
+        check(lib().dl_factor_bwd_directed(graph.ref, tg.ref, ptr(tperm), ptr(Z), ptr(G), ptr(kstar), ptr(w), ptr(s),
+                                           K, d, float(beta), one_minus(beta), float(T), ptr(dZ), ptr(r),
+                                           ptr(_x_scratch(graph)), ptr(routed), _optr(graph.hub_scratch(K * d)),
+                                           _optr(tg.hub_scratch(K * d)), stream_of(dev)), "dl_factor_bwd_directed")
+    return dZ, r
+
+
 class PairBatch:
     """A batch of (u,v) node pairs resident on the GPU (int32 ids), plus -- built lazily, once --
     the node-major incidence lists the atomic-free backward walks.
@@ -350,8 +374,12 @@ class _FactorAggregate(torch.autograd.Function):
     @staticmethod
     def backward(ctx, G, _gk, _gw, _gs):
         Z, kstar, w, s = ctx.saved_tensors
+        if ctx.graph.directed:
+            dZ, _ = factor_bwd_directed(ctx.graph, Z, G.contiguous(), kstar, w, s, ctx.beta, ctx.T)
+            return dZ, None, None, None
         # the gather-only backward collects the (j,i) terms from row i's side: it needs a symmetric
         # pattern (always true for adj_sym, main_disentangled.py:141-142).  Checked once per graph.
+        # A graph marked directed takes the backward over its transpose instead (above).
         ctx.graph.assert_symmetric()
         dZ, _ = factor_bwd(ctx.graph, Z, G.contiguous(), kstar, w, s, ctx.beta, ctx.T, sj=ctx.sj)
         return dZ, None, None, None
@@ -481,7 +509,7 @@ class _LinkBCELoss(torch.autograd.Function):
     def forward(ctx, Z, graph, batch, labels, weights, beta, T):
         Zc = Z.detach().contiguous()
         need_grad = ctx.needs_input_grad[0]        # False under torch.no_grad(): the eager backward is skipped
-        if need_grad:
+        if need_grad and not graph.directed:
             graph.assert_symmetric()          # gather-only backward (see _FactorAggregate.backward)
         kstar, w, s = edge_attn_fwd(graph, Zc, T)
         sj, zs = _spmm_side_buffers(graph, Zc, need_grad)
@@ -493,7 +521,10 @@ class _LinkBCELoss(torch.autograd.Function):
         loss, dS = link_bce(prob, labels, weights, want_grad=need_grad)
         if need_grad:
             dZ, dH = pair_score_bwd(Zc, H, batch, dS, T)
-            factor_bwd(graph, Zc, dH, kstar, w, s, beta, T, dZ=dZ, sj=sj)
+            if graph.directed:
+                factor_bwd_directed(graph, Zc, dH, kstar, w, s, beta, T, dZ=dZ)
+            else:
+                factor_bwd(graph, Zc, dH, kstar, w, s, beta, T, dZ=dZ, sj=sj)
             ctx.save_for_backward(dZ)
         ctx.mark_non_differentiable(prob, H)
         return loss, prob, H

@@ -548,11 +548,19 @@ class PartitionedLinkStep:
     Buffers are allocated once, rank-local.  The caller writes the factor embeddings of the nodes this
     rank owns into `self.Z_own` (a view of the first n_own rows of the local array) or passes them to
     `run()`; `run()` leaves dL/dZ of the owned rows in `self.dZ` ([n_own, K, d]), H of the owned rows in
-    `self.H[:n_own]` and all P scores in `self.prob`."""
+    `self.H[:n_own]` and all P scores in `self.prob`.
+
+    (src, dst) are the edge columns of an undirected graph: the step always trains on their symmetrisation
+    (adj_sym, see owned_entries).  ``directed=True`` -- training on the columns as given -- is refused: the
+    directed backward gathers over the transposed pattern on one GPU (ops.factor_bwd_directed) and has no
+    node-partitioned form."""
 
     def __init__(self, src, dst, n_global, u, v, labels, weights, K, d, beta, T,
                  world=1, rank=0, group=None, backend=None, device=None, mark=None, balance=True,
-                 peer_push=True, bounds=None):
+                 peer_push=True, bounds=None, directed=False):
+        if directed or getattr(src, "directed", False):
+            raise ValueError("PartitionedLinkStep trains on the symmetrised edge columns only: the directed "
+                             "backward (ops.factor_bwd_directed) runs on one GPU and has no node-partitioned form")
         self.mark = mark if mark is not None else (lambda name: None)  # phase boundary hook (bench)
         self.group = group
         self.be = backend if backend is not None else CudaBackend()

@@ -5,11 +5,16 @@ every per-epoch step on the device (negative sampling, fused BCE, AUC).
     python examples/train_link.py --dataset cora --root /path/to/reference/data --nfactor 3 --beta 0.9
     python examples/train_link.py --dataset chameleon --root /path/to/reference/data_pre_false --nfactor 5 --beta 0.7
     python examples/train_link.py --dataset synthetic
+    python examples/train_link.py --dataset chameleon --root /path/to/reference/data_pre_false --nfactor 5 --directed
 
 Same protocol as the script: 85/10/5 split of the directed edge columns, adjacency = symmetrised
 train edges, m rounds of structured negative sampling on the FULL edge set, loss = BCE(pos) +
 BCE(neg)/m over pairs that occur exactly once, early stopping on validation AUC computed from the
 training forward, test AUC with the best weights.
+
+--directed trains on the directed train adjacency (the script's ``adj``, main_disentangled.py:137-140) instead
+of ``adj_sym``: the train columns are used as given, in a graph marked directed, whose backward runs over the
+pattern and its transpose.  Split, negatives and AUC are unchanged.
 """
 from __future__ import annotations
 
@@ -59,7 +64,10 @@ def run(args, x, edge_index, device, log=print):
     E = edge_index.shape[1]
     tr, te, va = dl_data.split_edges(E, args.seed, device)
     train_edges = edge_index[:, tr]
-    graph = Graph.from_edges(train_edges[0], train_edges[1], n)            # adj_sym as a CSR
+    if getattr(args, "directed", False):                                   # adj as a CSR (:137-140)
+        graph = Graph.from_edges(train_edges[0], train_edges[1], n, directed=True)
+    else:
+        graph = Graph.from_edges(train_edges[0], train_edges[1], n)        # adj_sym as a CSR
     full = Graph.from_edges(edge_index[0], edge_index[1], n, symmetrize=False)
     edge_keys = torch.unique(edge_index[0] * n + edge_index[1])
     neg = {"tr": [], "va": [], "te": []}
@@ -131,6 +139,7 @@ def main():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--gpu", type=int, default=0)
     ap.add_argument("--log-every", type=int, default=10)
+    ap.add_argument("--directed", action="store_true", help="train on the directed train adjacency, not adj_sym")
     args = ap.parse_args()
     torch.manual_seed(args.seed)
     device = torch.device(f"cuda:{args.gpu}")

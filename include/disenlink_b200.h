@@ -82,6 +82,15 @@ int dl_csr_from_dense(const float* adj, int64_t N, int64_t* rowptr, int32_t* col
 int dl_rev_index(const int64_t* rowptr, const int32_t* col, int64_t N, int64_t nnz, int64_t* rev,
                  int32_t* status_out, dl_stream_t stream);
 
+/* Transposed pattern of a square CSR (the in-entries of every node), for the directed backward:
+ * trowptr [N+1], tcol [nnz] = source row of each in-entry, tperm [nnz] = CSR index of each in-entry.
+ * In-entries of a node are in CSR order (ascending source row for a CSR with sorted rows).  erow = the
+ * COO row array of the CSR (dl_entry_rows).  col must lie in [0,N); N, nnz < 2^31 - 1.  Integer work,
+ * bit-exact (stable radix sort). */
+size_t dl_transpose_index_workspace_bytes(int64_t N, int64_t nnz);
+int dl_transpose_index(const int32_t* col, const int32_t* erow, int64_t N, int64_t nnz, int64_t* trowptr,
+                       int32_t* tcol, int32_t* tperm, void* ws, size_t ws_bytes, dl_stream_t stream);
+
 /* Degree-sorted row bucketing: perm [N] = row ids ordered by degree class descending (stable),
  * bucket_off [DL_N_BUCKETS+1] (device int64) = start of each class in perm. */
 size_t dl_degree_buckets_workspace_bytes(int64_t N);
@@ -248,6 +257,21 @@ int dl_factor_bwd_edges(const dl_graph* g_host, const float* Z, const float* G,
                         const float* sj, float* sr_scratch, int64_t n_nodes, const float* x, int K,
                         int d, float one_minus_beta, float T, float* dZ, float* hub_ws,
                         dl_stream_t stream);
+/* Backward of the attention + aggregation for ANY 0/1 pattern (csrc/bwd_dir.cu): the autograd of
+ * model.py:56-75 when adj is not symmetric (e.g. the directed train adjacency).  Given G = dL/dH, with
+ * e = (i,j), k = kstar[e]:  T_[j,k] = (1-beta)/s[j,k] sum_{in-entries e of j, kstar=k} w[e] G[i,k];
+ * r[j,k] = <Z[j,k], T_[j,k]>/s[j,k], or 0 when row j has no entry routed to k (the reference's clamped
+ * s[j,k] = 1 passes no gradient); dZ[j] += beta G[j] + T_[j];  dw[e] = (1-beta)<G[i,k],Z[j,k]>/s[j,k] - r[i,k];
+ * coef[e,kk] = dw[e] w[e]/T ((kk==k) - a[e,kk]);  dZ[i,kk] += coef Z[j,kk];  dZ[j,kk] += coef Z[i,kk].
+ * g_host: the CSR (row_base 0, one GPU); gt_host, tperm: its transposed pattern as a dl_graph of its own
+ * (dl_transpose_index) and the CSR index of every in-entry.  dZ is accumulated into; r [N,K] is written.
+ * dw_scratch: nnz floats; routed_scratch: N uint32 (K <= 32); hub_ws / hub_ws_t:
+ * dl_hub_scratch_floats(g / gt, K*d) floats.  Gathers only, no floating-point atomics, deterministic. */
+int dl_factor_bwd_directed(const dl_graph* g_host, const dl_graph* gt_host, const int32_t* tperm,
+                           const float* Z, const float* G, const uint8_t* kstar, const float* w, const float* s,
+                           int K, int d, float beta, float one_minus_beta, float T, float* dZ, float* r,
+                           float* dw_scratch, uint32_t* routed_scratch, float* hub_ws, float* hub_ws_t,
+                           dl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * (5) factor-weighted link-pair scoring over explicit (u,v) batches.
