@@ -104,6 +104,10 @@ SIGNATURES = {
     "dl_link_bce": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp]),
     "dl_roc_auc_workspace_bytes": (_i64, [_i64]),
     "dl_roc_auc": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _vp]),
+    "dl_link_bce_segments_workspace_bytes": (_i64, [_i64]),
+    "dl_link_bce_segments": (_int, [_vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp]),
+    "dl_roc_auc_segments_workspace_bytes": (_i64, [_i64, _i64]),
+    "dl_roc_auc_segments": (_int, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp]),
     "dl_push_slice": (_int, [_vp, _vp, _int, _i64, _vp]),
     "dl_push_rows": (_int, [_vp, _i64, _int, _c.POINTER(DlPushDesc), _int, _vp]),
     "dl_need_masks": (_int, [_GP, _vp, _vp, _int, _vp, _vp]),

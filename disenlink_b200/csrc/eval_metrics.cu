@@ -121,6 +121,144 @@ __global__ void k_auc_final(const unsigned long long* __restrict__ acc, long lon
   out[4] = (double)acc[0];                                          // 2U (exact below 2^53)
 }
 
+// ---- per-segment AUC (dl_roc_auc_segments) ---------------------------------------------------------
+// The same statistic on every segment [seg_ptr[r], seg_ptr[r+1]) of one list.  Each element's key carries its
+// segment above the 32 score bits, so one stable radix sort orders the list by (segment, score): segment r's
+// elements then occupy exactly its own index range, and a tie group -- elements with equal 64-bit keys --
+// can never reach into a neighbouring segment even where the scores are equal.  The negative flags are
+// scanned once over the whole list; a positive subtracts the prefix at its segment's base.  Counts and 2U are
+// per-segment 64-bit integer sums (order-independent atomics), so each row equals dl_roc_auc on the segment
+// alone bit for bit.
+struct SegAucWs {
+  size_t key_a, key_b, lab_a, lab_b, negpre, acc, tmp, total;
+};
+
+SegAucWs seg_auc_ws_layout(long long P, long long R) {
+  SegAucWs w;
+  const size_t n = (size_t)(P > 0 ? P : 1);
+  const size_t a = dlp::sort_ws_bytes((long long)n), b = dlp::scan_ws_bytes((long long)n + 1, 4);
+  size_t off = 0;
+  w.key_a = off; off += ev_align256(n * 8);
+  w.key_b = off; off += ev_align256(n * 8);
+  w.lab_a = off; off += ev_align256(n);
+  w.lab_b = off; off += ev_align256(n);
+  w.negpre = off; off += ev_align256((n + 1) * 4);
+  w.acc = off; off += ev_align256((size_t)(R > 0 ? R : 1) * 3 * 8);   // u64 [3][R]: 2U, n_pos, n_nan
+  w.tmp = off; off += ev_align256(a > b ? a : b);
+  w.total = off;
+  return w;
+}
+
+// segment of element i: the largest r with seg_ptr[r] <= i (empty segments are skipped), clamped to [0, R)
+__device__ __forceinline__ int seg_of(const long long* __restrict__ seg_ptr, int R, long long i) {
+  int lo = 0, hi = R;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(seg_ptr + mid) <= i) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+
+// acc[seg] += v over the warp (all 32 lanes call it): one atomic when the warp sits in one segment
+__device__ __forceinline__ void seg_add(unsigned long long* acc, int seg, unsigned long long v) {
+  const int s0 = __shfl_sync(DL_FULL, seg, 0);
+  if (__all_sync(DL_FULL, seg == s0)) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(DL_FULL, v, o);
+    if ((threadIdx.x & 31) == 0 && v) atomicAdd(acc + s0, v);
+  } else if (v) {
+    atomicAdd(acc + seg, v);
+  }
+}
+
+__global__ void k_seg_auc_keys(const float* __restrict__ score, const float* __restrict__ labels, long long P,
+                               const long long* __restrict__ seg_ptr, int R,
+                               unsigned long long* __restrict__ key, unsigned char* __restrict__ lab,
+                               unsigned long long* __restrict__ acc) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i0 = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < P; i0 += stride) {
+    const long long i = i0 + (threadIdx.x & 31);
+    const bool valid = i < P;
+    const int seg = seg_of(seg_ptr, R, valid ? i : P - 1);
+    unsigned long long pos = 0, nan = 0;
+    if (valid) {
+      const float sc = __fadd_rn(__ldg(score + i), 0.0f);          // -0.0 -> +0.0
+      const unsigned b = __float_as_uint(sc);
+      const unsigned k = (b & 0x80000000u) ? ~b : (b | 0x80000000u); // ascending float order
+      key[i] = ((unsigned long long)seg << 32) | k;
+      const unsigned char l = __ldg(labels + i) != 0.0f;
+      lab[i] = l;
+      pos = l;
+      nan = (sc != sc);
+    }
+    seg_add(acc + R, seg, pos);
+    seg_add(acc + 2 * (long long)R, seg, nan);
+  }
+}
+
+struct NegFlagEnd {                    // scan input over P + 1 items: 1 for a negative, 0 past the end
+  const unsigned char* lab;
+  long long P;
+  __device__ __forceinline__ unsigned operator()(long long i) const { return (i < P && !lab[i]) ? 1u : 0u; }
+};
+
+__global__ void k_seg_auc_ranksum(const unsigned long long* __restrict__ key, const unsigned char* __restrict__ lab,
+                                  const unsigned* __restrict__ negpre, long long P,
+                                  const long long* __restrict__ seg_ptr, unsigned long long* __restrict__ acc) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i0 = (long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < P; i0 += stride) {
+    const long long i = i0 + (threadIdx.x & 31);
+    const unsigned long long k = key[i < P ? i : P - 1];
+    const int seg = (int)(k >> 32);
+    unsigned long long part = 0;
+    if (i < P && lab[i]) {
+      long long first = i, last = i;                               // tie group [first, last]: equal 64-bit keys
+      if (i > 0 && key[i - 1] == k) {                              // gallop left, then bisect
+        long long step = 1, hi = i;
+        long long lo = hi - step;
+        while (lo >= 0 && key[lo] == k) { hi = lo; step <<= 1; lo = hi - step; }
+        if (lo < -1) lo = -1;
+        while (hi - lo > 1) {
+          const long long mid = lo + (hi - lo) / 2;
+          if (key[mid] == k) hi = mid; else lo = mid;
+        }
+        first = hi;
+      }
+      if (i + 1 < P && key[i + 1] == k) {                          // gallop right
+        long long step = 1, lo = i;
+        long long hi = lo + step;
+        while (hi < P && key[hi] == k) { lo = hi; step <<= 1; hi = lo + step; }
+        if (hi > P) hi = P;
+        while (hi - lo > 1) {
+          const long long mid = lo + (hi - lo) / 2;
+          if (key[mid] == k) lo = mid; else hi = mid;
+        }
+        last = lo;
+      }
+      long long base = __ldg(seg_ptr + seg);
+      base = base < 0 ? 0 : (base > first ? first : base);
+      const unsigned long long nb = negpre[base];
+      part = (unsigned long long)(negpre[first] - nb) + (unsigned long long)(negpre[last + 1] - nb);
+    }
+    seg_add(acc, seg, part);
+  }
+}
+
+__global__ void k_seg_auc_final(const unsigned long long* __restrict__ acc, const long long* __restrict__ seg_ptr,
+                                int R, double* __restrict__ out) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= R) return;
+  const long long n = seg_ptr[r + 1] - seg_ptr[r];
+  const unsigned long long u2 = acc[r], pos = acc[R + r], nan = acc[2 * (long long)R + r];
+  const double npos = (double)pos, nneg = (double)((unsigned long long)n - pos);
+  const double nnan = (double)nan;
+  double auc = (double)u2 / (2.0 * npos * nneg);
+  if (npos == 0.0 || nneg == 0.0 || nnan != 0.0) auc = __longlong_as_double(0x7ff8000000000000LL);
+  double* o = out + 5 * (long long)r;
+  o[0] = auc; o[1] = npos; o[2] = nneg; o[3] = nnan;
+  o[4] = (double)u2;
+}
+
 }  // namespace
 
 extern "C" {
@@ -160,6 +298,49 @@ int dl_roc_auc(const float* score, const float* labels, int64_t P, double* out, 
     DL_LAUNCH_CHECK();
   }
   k_auc_final<<<1, 1, 0, st>>>(acc, P, out);
+  DL_LAUNCH_CHECK();
+  return DL_OK;
+}
+
+int64_t dl_roc_auc_segments_workspace_bytes(int64_t P, int64_t R) {
+  if (P < 0 || R < 1) return 0;
+  return (int64_t)seg_auc_ws_layout(P, R).total;
+}
+
+int dl_roc_auc_segments(const float* score, const float* labels, int64_t P, const int64_t* seg_ptr, int64_t R,
+                        double* out, void* ws, int64_t ws_bytes, dl_stream_t stream) {
+  if (P < 0 || P >= (1LL << 31) || R < 1 || R >= (1LL << 31) || !out || !seg_ptr ||
+      (P > 0 && (!score || !labels)))
+    return DL_EINVAL;
+  const SegAucWs w = seg_auc_ws_layout(P, R);
+  if (!ws || ws_bytes < (int64_t)w.total) return DL_EWORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  unsigned char* base = (unsigned char*)ws;
+  unsigned long long* key_a = (unsigned long long*)(base + w.key_a);
+  unsigned long long* key_b = (unsigned long long*)(base + w.key_b);
+  unsigned char* lab_a = base + w.lab_a;
+  unsigned char* lab_b = base + w.lab_b;
+  unsigned* negpre = (unsigned*)(base + w.negpre);
+  unsigned long long* acc = (unsigned long long*)(base + w.acc);
+  const long long* sp = (const long long*)seg_ptr;
+  DL_CUDA_TRY(cudaMemsetAsync(acc, 0, (size_t)R * 3 * 8, st));
+  if (P > 0) {
+    int seg_bits = 0;                                              // bits of the largest segment id, R - 1
+    while ((1LL << seg_bits) < R) ++seg_bits;
+    long long grid = (P + 255) / 256;
+    if (grid > 148 * 16) grid = 148 * 16;
+    k_seg_auc_keys<<<(int)grid, 256, 0, st>>>(score, labels, P, sp, (int)R, key_a, lab_a, acc);
+    DL_LAUNCH_CHECK();
+    int rc = dlp::sort_pairs<unsigned long long, unsigned char>(key_a, key_b, lab_a, lab_b, P, 0, 32 + seg_bits,
+                                                                base + w.tmp, st);
+    if (rc) return rc;
+    rc = dlp::scan<false, unsigned>(NegFlagEnd{lab_b, P}, dlp::StoreArr<unsigned>{negpre}, P + 1,
+                                    dlp::OpSum<unsigned>(), 0u, base + w.tmp, st);
+    if (rc) return rc;
+    k_seg_auc_ranksum<<<(int)grid, 256, 0, st>>>(key_b, lab_b, negpre, P, sp, acc);
+    DL_LAUNCH_CHECK();
+  }
+  k_seg_auc_final<<<(int)((R + 127) / 128), 128, 0, st>>>(acc, sp, (int)R, out);
   DL_LAUNCH_CHECK();
   return DL_OK;
 }

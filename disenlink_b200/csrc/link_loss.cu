@@ -13,6 +13,15 @@ namespace {
 
 constexpr int BCE_THREADS = 256;
 constexpr int BCE_MAX_BLOCKS = 148 * 8;
+constexpr int BCE_SEG_MAX_SLICES = 64;      // blocks per segment of dl_link_bce_segments
+
+// -w * (y log p + (1 - y) log(1 - p)) of one pair, logs clamped at -100 (torch's BCE)
+__device__ __forceinline__ float bce_term(float pr, float y, float wt) {
+  const float omp = __fsub_rn(1.0f, pr);
+  const float lp = fmaxf(logf(pr), -100.0f), lq = fmaxf(logf(omp), -100.0f);
+  const float term = __fadd_rn(__fmul_rn(y, lp), __fmul_rn(__fsub_rn(1.0f, y), lq));
+  return __fmul_rn(wt, term);
+}
 
 __global__ void __launch_bounds__(BCE_THREADS)
 k_link_bce(const float* __restrict__ prob, const float* __restrict__ labels,
@@ -24,9 +33,7 @@ k_link_bce(const float* __restrict__ prob, const float* __restrict__ labels,
     const float pr = __ldg(prob + p), y = __ldg(labels + p);
     const float wt = weights ? __ldg(weights + p) : 1.0f;
     const float omp = __fsub_rn(1.0f, pr);
-    const float lp = fmaxf(logf(pr), -100.0f), lq = fmaxf(logf(omp), -100.0f);
-    const float term = __fadd_rn(__fmul_rn(y, lp), __fmul_rn(__fsub_rn(1.0f, y), lq));
-    acc -= (double)__fmul_rn(wt, term);
+    acc -= (double)bce_term(pr, y, wt);
     if (dS) {
       const float pq = __fmul_rn(omp, pr);
       const float dprob = __fdiv_rn(__fmul_rn(wt, __fsub_rn(pr, y)), fmaxf(pq, 1e-12f));
@@ -55,6 +62,52 @@ __global__ void __launch_bounds__(32) k_link_bce_final(const double* __restrict_
   if (threadIdx.x == 0) *loss = (float)acc;
 }
 
+// Segment r = blockIdx.x, slice blockIdx.y of gridDim.y: a block-stride walk over the segment, partial sums
+// in double, reduced in a fixed order into partial[r * slices + slice].
+__global__ void __launch_bounds__(BCE_THREADS)
+k_link_bce_seg(const float* __restrict__ prob, const float* __restrict__ labels,
+               const float* __restrict__ weights, long long P, const long long* __restrict__ seg_ptr,
+               double* __restrict__ partial) {
+  const long long r = blockIdx.x;
+  long long lo = __ldg(seg_ptr + r), hi = __ldg(seg_ptr + r + 1);
+  lo = lo < 0 ? 0 : (lo > P ? P : lo);                 // a malformed seg_ptr cannot read outside [0, P)
+  hi = hi < lo ? lo : (hi > P ? P : hi);
+  double acc = 0.0;
+  const long long stride = (long long)gridDim.y * BCE_THREADS;
+  for (long long p = lo + (long long)blockIdx.y * BCE_THREADS + threadIdx.x; p < hi; p += stride) {
+    const float wt = weights ? __ldg(weights + p) : 1.0f;
+    acc -= (double)bce_term(__ldg(prob + p), __ldg(labels + p), wt);
+  }
+  __shared__ double red[BCE_THREADS / 32];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(DL_FULL, acc, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+#pragma unroll
+    for (int i = 0; i < BCE_THREADS / 32; ++i) t += red[i];
+    partial[r * gridDim.y + blockIdx.y] = t;
+  }
+}
+
+// one warp per segment sums its slices in a fixed order
+__global__ void __launch_bounds__(BCE_THREADS)
+k_link_bce_seg_final(const double* __restrict__ partial, int slices, long long R, float* __restrict__ loss) {
+  const long long r = (long long)blockIdx.x * (BCE_THREADS / 32) + (threadIdx.x >> 5);
+  if (r >= R) return;                                  // warp-uniform
+  double acc = 0.0;
+  for (int i = threadIdx.x & 31; i < slices; i += 32) acc += partial[r * slices + i];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(DL_FULL, acc, o);
+  if ((threadIdx.x & 31) == 0) loss[r] = (float)acc;
+}
+
+int bce_seg_slices(long long R) {
+  long long s = BCE_MAX_BLOCKS / (R > 0 ? R : 1);
+  return (int)(s < 1 ? 1 : (s > BCE_SEG_MAX_SLICES ? BCE_SEG_MAX_SLICES : s));
+}
+
 }  // namespace
 
 extern "C" {
@@ -72,6 +125,27 @@ int dl_link_bce(const float* prob, const float* labels, const float* weights, in
   k_link_bce<<<(int)grid, BCE_THREADS, 0, st>>>(prob, labels, weights, P, dS, (double*)ws);
   DL_LAUNCH_CHECK();
   k_link_bce_final<<<1, 32, 0, st>>>((const double*)ws, (int)grid, loss);
+  DL_LAUNCH_CHECK();
+  return DL_OK;
+}
+
+int64_t dl_link_bce_segments_workspace_bytes(int64_t R) {
+  if (R < 1) return 0;
+  return R * (int64_t)bce_seg_slices(R) * (int64_t)sizeof(double);
+}
+
+int dl_link_bce_segments(const float* prob, const float* labels, const float* weights, int64_t P,
+                         const int64_t* seg_ptr, int64_t R, float* loss, void* ws, int64_t ws_bytes,
+                         dl_stream_t stream) {
+  if (P < 0 || R < 1 || R >= (1LL << 31) || !loss || !seg_ptr || (P > 0 && (!prob || !labels))) return DL_EINVAL;
+  if (!ws || ws_bytes < dl_link_bce_segments_workspace_bytes(R)) return DL_EWORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int slices = bce_seg_slices(R);
+  k_link_bce_seg<<<dim3((unsigned)R, (unsigned)slices), BCE_THREADS, 0, st>>>(prob, labels, weights, P,
+                                                                              (const long long*)seg_ptr, (double*)ws);
+  DL_LAUNCH_CHECK();
+  const long long per = BCE_THREADS / 32;
+  k_link_bce_seg_final<<<(unsigned)((R + per - 1) / per), BCE_THREADS, 0, st>>>((const double*)ws, slices, R, loss);
   DL_LAUNCH_CHECK();
   return DL_OK;
 }

@@ -489,6 +489,76 @@ def roc_auc_stats(score, labels):
     return out
 
 
+def _check_seg_ptr(seg_ptr, device) -> int:
+    """-> R.  seg_ptr must be an int64 [R+1] tensor on `device`; its values (0 = seg_ptr[0] <= ... <=
+    seg_ptr[R] = P) are not read back here, which would synchronise with the device."""
+    require_cuda(seg_ptr, "seg_ptr")
+    if seg_ptr.dtype != torch.int64 or seg_ptr.dim() != 1 or seg_ptr.numel() < 2:
+        raise ValueError("seg_ptr must be an int64 tensor [R+1] with R >= 1")
+    if seg_ptr.device != device:
+        raise ValueError(f"seg_ptr is on {seg_ptr.device}, the scores on {device}")
+    return int(seg_ptr.numel()) - 1
+
+
+def _check_per_pair(t, name, device, P: int):
+    """A per-pair input of the segmented calls: on `device`, P elements (it is read through a raw pointer)."""
+    if t.device != device:
+        raise ValueError(f"{name} is on {t.device}, the scores on {device}")
+    if t.numel() != P:
+        raise ValueError(f"{name} has {t.numel()} elements, the scores {P}")
+
+
+def roc_auc_segments(score, labels, seg_ptr):
+    """roc_auc_stats of every segment [seg_ptr[r], seg_ptr[r+1]) of one score list in one launch sequence:
+    -> float64 tensor [R, 5] on the device, row r = (auc, n_pos, n_neg, n_nan, 2U) of segment r alone (see
+    dl_roc_auc_segments).  Equal scores in different segments never tie.  No host sync."""
+    dev = score.device
+    require_cuda(score, "score")
+    if score.dtype != torch.float32:
+        raise TypeError("score must be float32")
+    P = int(score.numel())
+    R = _check_seg_ptr(seg_ptr, dev)
+    _check_per_pair(labels, "labels", dev, P)
+    score = score.contiguous()
+    labels = labels.to(torch.float32).contiguous()
+    L = lib()
+    with torch.cuda.device(dev):
+        out = torch.empty(R, 5, dtype=torch.float64, device=dev)
+        ws_bytes = int(L.dl_roc_auc_segments_workspace_bytes(P, R))
+        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+        check(L.dl_roc_auc_segments(ptr(score), ptr(labels), P, ptr(seg_ptr.contiguous()), R, ptr(out), ptr(ws),
+                                    ws_bytes, stream_of(dev)), "dl_roc_auc_segments")
+    return out
+
+
+def link_bce_segments(prob, labels, weights, seg_ptr):
+    """The loss of link_bce on every segment [seg_ptr[r], seg_ptr[r+1]) of one pair list -> float32 [R] on the
+    device (an empty segment gives 0).  Loss only: the gradient of the whole list comes from link_bce /
+    link_bce_loss.  `weights` may be None (all ones).  No host sync."""
+    dev = prob.device
+    require_cuda(prob, "prob")
+    if prob.dtype != torch.float32:
+        raise TypeError("prob must be float32")
+    P = int(prob.numel())
+    R = _check_seg_ptr(seg_ptr, dev)
+    _check_per_pair(labels, "labels", dev, P)
+    if weights is not None:
+        _check_per_pair(weights, "weights", dev, P)
+    prob = prob.contiguous()
+    labels = labels.to(torch.float32).contiguous()
+    if weights is not None:
+        weights = weights.to(torch.float32).contiguous()
+    L = lib()
+    with torch.cuda.device(dev):
+        loss = torch.empty(R, dtype=torch.float32, device=dev)
+        ws_bytes = int(L.dl_link_bce_segments_workspace_bytes(R))
+        ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+        check(L.dl_link_bce_segments(ptr(prob), ptr(labels), ptr(weights) if weights is not None else None, P,
+                                     ptr(seg_ptr.contiguous()), R, ptr(loss), ptr(ws), ws_bytes, stream_of(dev)),
+              "dl_link_bce_segments")
+    return loss
+
+
 def roc_auc(score, labels) -> float:
     """sklearn.metrics.roc_auc_score(labels, score) for binary labels, computed on the device
     (main_disentangled.py:204,219).  Raises ValueError where sklearn does (one class only, NaN)."""

@@ -15,6 +15,11 @@ training forward, test AUC with the best weights.
 --directed trains on the directed train adjacency (the script's ``adj``, main_disentangled.py:137-140) instead
 of ``adj_sym``: the train columns are used as given, in a graph marked directed, whose backward runs over the
 pattern and its transpose.  Split, negatives and AUC are unchanged.
+
+--run R (main_disentangled.py:131,224) trains R independent runs with seeds --seed, --seed + 1, ... together:
+one union graph, one stacked model, one optimizer step per epoch (disenlink_b200/runs.py), per-run early
+stopping, then the per-run test AUCs and their mean +- std.  Run r gives what a single run with
+--seed (seed + r) gives, up to the summation order of the batched GEMMs.
 """
 from __future__ import annotations
 
@@ -23,6 +28,7 @@ import copy
 import os
 import sys
 
+import numpy as np
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -30,6 +36,7 @@ from disenlink_b200 import data as dl_data  # noqa: E402
 from disenlink_b200 import ops  # noqa: E402
 from disenlink_b200.graph import Graph  # noqa: E402
 from disenlink_b200.model import Disentangle  # noqa: E402
+from disenlink_b200.runs import DisentangleRuns, EarlyStopping, RunSet, edge_labels  # noqa: E402
 
 
 def synthetic(n=3000, communities=8, deg=12, feat=64, seed=0):
@@ -48,13 +55,6 @@ def synthetic(n=3000, communities=8, deg=12, feat=64, seed=0):
     x = torch.nn.functional.one_hot(comm, communities).float() @ torch.randn(communities, feat, generator=g)
     x = x + 0.5 * torch.randn(n, feat, generator=g)
     return x, torch.stack([key // n, key % n]), comm
-
-
-def edge_labels(u, v, edge_keys, n):
-    """ori_adj[u, v] of the script: 1 where (u, v) is a column of the full edge set."""
-    k = u.long() * n + v.long()
-    pos = torch.searchsorted(edge_keys, k).clamp_(max=edge_keys.numel() - 1)
-    return (edge_keys[pos] == k).float()
 
 
 def run(args, x, edge_index, device, log=print):
@@ -123,6 +123,73 @@ def run(args, x, edge_index, device, log=print):
     return {"history": history, "best_val_auc": best_auc, "test_auc": test_auc}
 
 
+def batched_model(args, nfeat, seeds):
+    """DisentangleRuns whose run r is the model run() builds after torch.manual_seed(seeds[r])."""
+    models = []
+    for seed in seeds:
+        torch.manual_seed(seed)
+        models.append(Disentangle(nfeat, args.nhidden, args.nembed, nfactor=args.nfactor, beta=args.beta,
+                                  t=args.temperature))
+    return DisentangleRuns.from_models(models)
+
+
+def batched_epoch(args, x, runs, model, opt, stop):
+    """One epoch of every run: projection, fused loss forward + backward over the union, one Adam step, the
+    per-run losses and validation AUCs, the stopping update.  -> host list [R losses, R AUCs, R best AUCs,
+    R stopped flags], the epoch's one device-to-host copy."""
+    Z = model.project(x)
+    loss, prob, H = ops.link_bce_loss(Z, runs.graph, runs.train, runs.train_labels, runs.train_weights,
+                                      args.beta, args.temperature)
+    opt.zero_grad()
+    loss.backward()
+    opt.step()
+    run_loss = ops.link_bce_segments(prob, runs.train_labels, runs.train_weights, runs.train_ptr)
+    _, val_prob = ops.pair_score_fwd(Z.detach(), H, runs.val, args.temperature, want_logit=False)
+    auc = ops.roc_auc_segments(val_prob, runs.val_labels, runs.val_ptr)[:, 0]
+    stop.update(auc)
+    return torch.cat([run_loss.double(), auc, stop.best_auc, stop.stopped.double()]).cpu().tolist()
+
+
+def run_batched(args, x, edge_index, device, log=print):
+    """run() for seeds args.seed + r, r < args.run, trained together (main_disentangled.py:131-224).
+    -> {"runs": [{"seed", "history", "best_val_auc", "test_auc"} per run], "test_auc_mean", "test_auc_std"}"""
+    n = x.shape[0]
+    x = dl_data.row_standardize(x).to(device) if args.standardize else x.to(device)
+    seeds = [args.seed + r for r in range(args.run)]
+    runs = RunSet(edge_index.to(device), n, seeds, args.m, directed=getattr(args, "directed", False))
+    model = batched_model(args, x.shape[1], seeds).to(device)
+    opt = torch.optim.Adam(model.parameters(), lr=args.lr, weight_decay=5e-4)
+    stop = EarlyStopping(list(model.parameters()), patience=200)
+    R = len(seeds)
+    history = [[] for _ in range(R)]
+    active = [True] * R
+    for epoch in range(args.epochs):
+        host = batched_epoch(args, x, runs, model, opt, stop)
+        for r in range(R):
+            if active[r]:
+                history[r].append((host[r], host[R + r]))
+        active = [not bool(f) for f in host[3 * R:]]
+        if epoch % args.log_every == 0:
+            log(f"epoch: {epoch} active runs: {sum(active)}/{R} loss: {np.mean(host[:R]):.5f} (mean) "
+                f"val_auc: " + " ".join(f"{b:.4f}" for b in host[2 * R:3 * R]))
+        if not any(active):
+            break
+    stop.restore()
+    with torch.no_grad():
+        Z = model.project(x)
+        H = ops.factor_aggregate(Z, runs.graph, args.beta, args.temperature)
+        _, test_prob = ops.pair_score_fwd(Z, H, runs.test, args.temperature, want_logit=False)
+    test_auc = ops.roc_auc_segments(test_prob, runs.test_labels, runs.test_ptr)[:, 0].tolist()
+    best_val = stop.best_auc.tolist()
+    out = []
+    for r, seed in enumerate(seeds):
+        log(f"run {r} (seed {seed}): epochs {len(history[r])} best val auc {best_val[r]:.4f} test auc {test_auc[r]:.4f}")
+        out.append({"seed": seed, "history": history[r], "best_val_auc": best_val[r], "test_auc": test_auc[r]})
+    mean, std = float(np.mean(test_auc)), float(np.std(test_auc))
+    log(f"test auc over {R} runs: {mean:.4f} ± {std:.4f}")
+    return {"runs": out, "test_auc_mean": mean, "test_auc_std": std}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--dataset", default="synthetic")
@@ -140,7 +207,10 @@ def main():
     ap.add_argument("--gpu", type=int, default=0)
     ap.add_argument("--log-every", type=int, default=10)
     ap.add_argument("--directed", action="store_true", help="train on the directed train adjacency, not adj_sym")
+    ap.add_argument("--run", type=int, default=1, help="independent runs (seeds --seed + r), trained together")
     args = ap.parse_args()
+    if args.run < 1:
+        ap.error(f"--run must be >= 1, got {args.run}")
     torch.manual_seed(args.seed)
     device = torch.device(f"cuda:{args.gpu}")
     if args.dataset in ("cora", "citeseer", "pubmed"):
@@ -162,7 +232,10 @@ def main():
     else:
         x, edge_index, _ = synthetic(seed=args.seed)
         args.standardize = True
-    run(args, x, edge_index, device)
+    if args.run > 1:
+        run_batched(args, x, edge_index, device)
+    else:
+        run(args, x, edge_index, device)
 
 
 if __name__ == "__main__":

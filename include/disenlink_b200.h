@@ -332,6 +332,19 @@ int64_t dl_link_bce_workspace_bytes(void);
 int dl_link_bce(const float* prob, const float* labels, const float* weights, int64_t P, float* dS,
                 float* loss, void* ws, int64_t ws_bytes, dl_stream_t stream);
 
+/* The loss of dl_link_bce on every segment [seg_ptr[r], seg_ptr[r+1]) of one pair list, r < R: the independent
+ * runs of the script trained as one union (disenlink_b200/runs.py), each run's pairs one segment.
+ * [ref: main_disentangled.py:131,195 -- one loss per run of the `for run in range(args.run)` loop]
+ *   loss[r] = sum over the segment of weights[p] * -( y log p + (1 - y) log(1 - p) )   (dl_link_bce's terms)
+ * Loss only (the gradient of the union comes from dl_link_bce).  seg_ptr: int64 [R+1] on the device,
+ * 0 = seg_ptr[0] <= ... <= seg_ptr[R] = P (reads are clamped to [0, P) whatever it holds); an empty segment
+ * gives 0.  Deterministic: double partial sums combined in a fixed order.
+ * ws: >= dl_link_bce_segments_workspace_bytes(R) bytes of device scratch. */
+int64_t dl_link_bce_segments_workspace_bytes(int64_t R);
+int dl_link_bce_segments(const float* prob, const float* labels, const float* weights, int64_t P,
+                         const int64_t* seg_ptr, int64_t R, float* loss, void* ws, int64_t ws_bytes,
+                         dl_stream_t stream);
+
 /* ---- ROC-AUC of a score list ----------------------------------------------------------------
  * [ref: main_disentangled.py:202-204,217-219 -- sklearn.metrics.roc_auc_score(y, a_pred[mask == 1])]
  * labels: 0 / non-zero floats.  out: 5 doubles on the device = { auc, n_pos, n_neg, n_nan, 2U } where
@@ -341,6 +354,16 @@ int dl_link_bce(const float* prob, const float* labels, const float* weights, in
 int64_t dl_roc_auc_workspace_bytes(int64_t P);
 int dl_roc_auc(const float* score, const float* labels, int64_t P, double* out, void* ws, int64_t ws_bytes,
                dl_stream_t stream);
+
+/* dl_roc_auc on every segment [seg_ptr[r], seg_ptr[r+1]) of one score list, r < R: out[5r .. 5r+4] =
+ * { auc, n_pos, n_neg, n_nan, 2U } of that segment alone, equal bit for bit to dl_roc_auc on it (an empty,
+ * one-class or NaN segment gives NaN in its own row only).  Equal scores in different segments never tie.
+ * [ref: main_disentangled.py:131,202-204,217-219 -- roc_auc_score per run of the `for run in range(args.run)` loop]
+ * seg_ptr: int64 [R+1] on the device with 0 = seg_ptr[0] <= ... <= seg_ptr[R] = P.  P < 2^31, 1 <= R < 2^31.
+ * ws: >= dl_roc_auc_segments_workspace_bytes(P, R) bytes of device scratch. */
+int64_t dl_roc_auc_segments_workspace_bytes(int64_t P, int64_t R);
+int dl_roc_auc_segments(const float* score, const float* labels, int64_t P, const int64_t* seg_ptr, int64_t R,
+                        double* out, void* ws, int64_t ws_bytes, dl_stream_t stream);
 
 /* ---- structured negative sampling ---------------------------------------------------------
  * [ref: main_disentangled.py:160 -- torch_geometric.utils.structured_negative_sampling(edge_index)]
