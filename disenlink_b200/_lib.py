@@ -91,6 +91,8 @@ SIGNATURES = {
     "dl_factor_bwd_edges": (_int, [_GP, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _int, _int, _f, _f, _vp, _vp, _vp]),
     "dl_factor_bwd_directed": (_int, [_GP, _GP, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _f, _f, _f, _vp, _vp, _vp, _vp,
                                       _vp, _vp, _vp]),
+    "dl_factor_bwd_directed_phase": (_int, [_GP, _GP, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _f, _f, _f, _i64, _i64,
+                                            _vp, _vp, _vp, _vp, _vp, _vp, _int, _vp]),
     "dl_pair_score_fwd": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _int, _int, _f, _vp, _vp, _vp]),
     "dl_pair_incidence_workspace_bytes": (_sz, [_i64, _i64]),
     "dl_pair_incidence": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -110,6 +112,7 @@ SIGNATURES = {
     "dl_roc_auc_segments": (_int, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _i64, _vp]),
     "dl_push_slice": (_int, [_vp, _vp, _int, _i64, _vp]),
     "dl_push_rows": (_int, [_vp, _i64, _int, _c.POINTER(DlPushDesc), _int, _vp]),
+    "dl_push_entries": (_int, [_vp, _int, _c.POINTER(DlPushDesc), _int, _vp]),
     "dl_need_masks": (_int, [_GP, _vp, _vp, _int, _vp, _vp]),
     "dl_factor_spmm_fwd_push": (_int, [_GP, _vp, _vp, _vp, _vp, _int, _int, _f, _f, _vp, _vp, _vp, _vp, _int, _vp]),
     "dl_edge_attn_fwd_push": (_int, [_GP, _vp, _int, _int, _f, _vp, _vp, _vp, _vp, _vp, _int, _vp]),

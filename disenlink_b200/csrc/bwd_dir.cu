@@ -268,6 +268,49 @@ int launch_dir_edges(const DlGraphDev& g, const int* tperm, const float* Z, cons
   return DL_OK;
 }
 
+// the three phases of the directed backward; arguments validated by the caller
+int dir_phase(const DlGraphDev& g, const DlGraphDev& gt, const int32_t* tperm, const float* Z, const float* G,
+              const uint8_t* kstar, const float* w, const float* s, int K, int d, float beta, float omb, float T,
+              float* dZ, float* r, float* dw, uint32_t* routed, float* hub_ws, float* hub_ws_t, int phase,
+              cudaStream_t st) {
+  int grid = 1, rc = DL_OK;
+  switch (phase) {
+    case 1:
+      rc = dl_grid_for(k_routed_mask, g.N, &grid);
+      if (rc) return rc;
+      k_routed_mask<<<grid, DL_CTA, 0, st>>>(g, kstar, routed);
+      DL_LAUNCH_CHECK();
+      rc = dl_grid_for(k_dir_gather, gt.n_hub_items + (gt.N - gt.n_hub), &grid);
+      if (rc) return rc;
+      k_dir_gather<<<grid, DL_CTA, 0, st>>>(gt, tperm, Z, G, kstar, w, s, routed, K, d, beta, omb, dZ, r, hub_ws_t);
+      DL_LAUNCH_CHECK();
+      if (gt.n_hub > 0) {
+        rc = dl_grid_for(k_dir_gather_hub, gt.n_hub, &grid);
+        if (rc) return rc;
+        k_dir_gather_hub<<<grid, DL_CTA, 0, st>>>(gt, Z, G, s, routed, K, d, beta, omb, dZ, r, hub_ws_t);
+        DL_LAUNCH_CHECK();
+      }
+      return DL_OK;
+    case 2:
+      return launch_dir_edges<false>(g, nullptr, Z, G, kstar, s, r, K, d, omb, T, dw, dZ, hub_ws, st);
+    case 3:
+      return launch_dir_edges<true>(gt, tperm, Z, G, kstar, s, r, K, d, omb, T, dw, dZ, hub_ws_t, st);
+    default:
+      return DL_EINVAL;
+  }
+}
+
+// status |= 1 when some index of a[0, n) is outside [0, bound)
+__global__ void k_dir_bounds(const int32_t* __restrict__ a, long long n, long long bound, int* __restrict__ status) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  bool bad = false;
+  for (long long x = (long long)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += stride) {
+    const int v = __ldg(a + x);
+    bad |= v < 0 || (long long)v >= bound;
+  }
+  if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(status, 1);
+}
+
 }  // namespace
 
 extern "C" {
@@ -288,27 +331,58 @@ int dl_factor_bwd_directed(const dl_graph* g_host, const dl_graph* gt_host, cons
   cudaStream_t st = (cudaStream_t)stream;
   const DlGraphDev g = dl_graph_dev(g_host);
   const DlGraphDev gt = dl_graph_dev(gt_host);
-  int grid = 1;
-  int rc = dl_grid_for(k_routed_mask, g.N, &grid);
-  if (rc) return rc;
-  k_routed_mask<<<grid, DL_CTA, 0, st>>>(g, kstar, routed_scratch);
-  DL_LAUNCH_CHECK();
-  rc = dl_grid_for(k_dir_gather, gt.n_hub_items + (gt.N - gt.n_hub), &grid);
-  if (rc) return rc;
-  k_dir_gather<<<grid, DL_CTA, 0, st>>>(gt, tperm, Z, G, kstar, w, s, routed_scratch, K, d, beta, one_minus_beta,
-                                        dZ, r, hub_ws_t);
-  DL_LAUNCH_CHECK();
-  if (gt.n_hub > 0) {
-    rc = dl_grid_for(k_dir_gather_hub, gt.n_hub, &grid);
+  for (int phase = 1; phase <= 3; ++phase) {
+    const int rc = dir_phase(g, gt, tperm, Z, G, kstar, w, s, K, d, beta, one_minus_beta, T, dZ, r, dw_scratch,
+                             routed_scratch, hub_ws, hub_ws_t, phase, st);
     if (rc) return rc;
-    k_dir_gather_hub<<<grid, DL_CTA, 0, st>>>(gt, Z, G, s, routed_scratch, K, d, beta, one_minus_beta, dZ, r,
-                                              hub_ws_t);
-    DL_LAUNCH_CHECK();
   }
-  rc = launch_dir_edges<false>(g, nullptr, Z, G, kstar, s, r, K, d, one_minus_beta, T, dw_scratch, dZ, hub_ws, st);
-  if (rc) return rc;
-  return launch_dir_edges<true>(gt, tperm, Z, G, kstar, s, r, K, d, one_minus_beta, T, dw_scratch, dZ, hub_ws_t,
-                                st);
+  return DL_OK;
+}
+
+int dl_factor_bwd_directed_phase(const dl_graph* g_host, const dl_graph* gt_host, const int32_t* tperm,
+                                 const float* Z, const float* G, const uint8_t* kstar, const float* w,
+                                 const float* s, int K, int d, float beta, float one_minus_beta, float T,
+                                 int64_t n_tot, int64_t n_rec, float* dZ, float* r, float* dw,
+                                 uint32_t* routed_scratch, float* hub_ws, float* hub_ws_t, int phase,
+                                 dl_stream_t stream) {
+  if (phase < 1 || phase > 3) return DL_EINVAL;
+  if (!dl_graph_ok(g_host) || !dl_graph_ok(gt_host) || !dl_shape_ok(K, d)) return DL_EINVAL;
+  if (gt_host->N != g_host->N || g_host->row_base != 0 || gt_host->row_base != 0) return DL_EINVAL;
+  if (n_tot < g_host->N || n_tot >= (1LL << 31) || n_rec < g_host->nnz || n_rec >= (1LL << 31)) return DL_EINVAL;
+  if (!(T == T) || T == 0.0f) return DL_EINVAL;
+  if (g_host->N == 0) return DL_OK;
+  const bool out_side = phase != 3, in_side = phase != 2;
+  if (!Z || !dZ || (phase != 3 && (!G || !s || !r)) || (phase == 1 && !routed_scratch)) return DL_EINVAL;
+  if ((out_side && g_host->nnz > 0 && !kstar) || (in_side && gt_host->nnz > 0 && (!kstar || !tperm))) return DL_EINVAL;
+  if ((phase == 1 && gt_host->nnz > 0 && !w) || (phase == 2 && g_host->nnz > 0 && !dw) ||
+      (phase == 3 && gt_host->nnz > 0 && !dw))
+    return DL_EINVAL;
+  if ((phase == 2 && g_host->n_hub_items > 0 && !hub_ws) || (in_side && gt_host->n_hub_items > 0 && !hub_ws_t))
+    return DL_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  const DlGraphDev g = dl_graph_dev(g_host);
+  const DlGraphDev gt = dl_graph_dev(gt_host);
+  // the phase's column and record indices against n_tot / n_rec: one pass and one synchronisation
+  const long long n_g = phase == 2 ? g.nnz : 0, n_t = in_side ? gt.nnz : 0;
+  if (n_g + n_t > 0) {
+    int* status = nullptr;
+    DL_CUDA_TRY(cudaMallocAsync((void**)&status, sizeof(int), st));
+    DL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(int), st));
+    if (n_g > 0) k_dir_bounds<<<fixup_blocks(n_g), 256, 0, st>>>(g.col, n_g, n_tot, status);
+    if (n_t > 0) {
+      k_dir_bounds<<<fixup_blocks(n_t), 256, 0, st>>>(gt.col, n_t, n_tot, status);
+      k_dir_bounds<<<fixup_blocks(n_t), 256, 0, st>>>(tperm, n_t, n_rec, status);
+    }
+    int bad = 0;
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&bad, status, sizeof(int), cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(status, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return (int)e;
+    if (bad) return DL_EINVAL;
+  }
+  return dir_phase(g, gt, tperm, Z, G, kstar, w, s, K, d, beta, one_minus_beta, T, dZ, r, dw, routed_scratch, hub_ws,
+                   hub_ws_t, phase, st);
 }
 
 }  // extern "C"

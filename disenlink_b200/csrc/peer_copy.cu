@@ -201,6 +201,56 @@ extern "C" int dl_need_masks(const dl_graph* g_host, const uint8_t* kstar, const
   return DL_OK;
 }
 
+// ---- per-entry records of the directed step (kstar, w, dw): the owner of an entry pushes it to the owner of its
+// column.  Elements of 1 or 4 bytes, one thread per (element, peer), peers inner so consecutive stores of a warp
+// alternate destinations like k_push_rows.
+namespace {
+
+template <typename E>
+__global__ void __launch_bounds__(256)
+k_push_entries(const E* __restrict__ src, int n_peers, long long most, const __grid_constant__ PushTable tab) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < most; t += stride) {
+#pragma unroll 1
+    for (int q = 0; q < n_peers; ++q) {
+      const dl_push_desc& d = tab.d[q];
+      if (t >= d.n) continue;
+      const long long sr = d.src_idx ? (long long)__ldg(d.src_idx + t) : t;
+      const long long dr = d.dst_idx ? (long long)__ldg(d.dst_idx + t) : t;
+      reinterpret_cast<E*>(d.dst)[dr] = __ldg(src + sr);
+    }
+  }
+}
+
+}  // namespace
+
+extern "C" int dl_push_entries(const void* src, int elem_bytes, const dl_push_desc* descs_host, int n_peers,
+                               dl_stream_t stream) {
+  if (n_peers < 0 || n_peers > DL_MAX_PEERS || (elem_bytes != 1 && elem_bytes != 4)) return DL_EINVAL;
+  if (n_peers == 0) return DL_OK;
+  if (!descs_host) return DL_EINVAL;
+  PushTable tab;
+  long long most = 0;
+  for (int q = 0; q < n_peers; ++q) {
+    tab.d[q] = descs_host[q];
+    const dl_push_desc& d = tab.d[q];
+    if (d.n < 0 || d.mask) return DL_EINVAL;
+    if (d.n > 0 && (!d.dst || ((uintptr_t)d.dst & (elem_bytes - 1)) != 0)) return DL_EINVAL;
+    if (d.n > most) most = d.n;
+  }
+  if (most == 0) return DL_OK;
+  if (!src || ((uintptr_t)src & (elem_bytes - 1)) != 0) return DL_EINVAL;
+  long long grid = (most + 255) / 256;
+  if (grid > 148LL * 8) grid = 148LL * 8;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (elem_bytes == 1)
+    k_push_entries<unsigned char><<<(unsigned)grid, 256, 0, st>>>((const unsigned char*)src, n_peers, most, tab);
+  else
+    k_push_entries<unsigned><<<(unsigned)grid, 256, 0, st>>>((const unsigned*)src, n_peers, most, tab);
+  DL_LAUNCH_CHECK();
+  return DL_OK;
+}
+
 // enable stores from the current device into `peer_device`'s memory (idempotent)
 extern "C" int dl_enable_peer_access(int peer_device) {
   int cur = 0, can = 0;

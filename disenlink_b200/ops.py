@@ -263,6 +263,46 @@ def factor_bwd_directed(graph: Graph, Z, G, kstar, w, s, beta: float, T: float =
     return dZ, r
 
 
+def factor_bwd_directed_phase(graph: Graph, tgraph: Graph, tperm, Z, G, kstar, w, s, beta: float, T: float, dZ, r,
+                              dw, routed, phase: int):
+    """One phase of factor_bwd_directed (dl_factor_bwd_directed_phase) on rank-local graphs: 1 = pass 1 over the
+    in-entries (r, dZ += beta G + T_), 2 = pass 2 out-side (writes dw of the own entries), 3 = pass 2 in-side
+    (reads kstar, dw through tperm).  `graph` / `tgraph`: the owned rows and their in-entries (same N, row_base 0),
+    columns below Z.shape[0]; kstar, w, dw: the per-entry records [own entries | records of remote in-entries],
+    every tperm value below their length.  `routed`: int32 [N] scratch of phase 1."""
+    K, d = int(Z.shape[1]), int(Z.shape[2])
+    dev = Z.device
+    n_rec = min(int(kstar.numel()), int(dw.numel()) if dw is not None else 1 << 62,
+                int(w.numel()) if w is not None else 1 << 62)
+    with torch.cuda.device(dev):
+        check(lib().dl_factor_bwd_directed_phase(graph.ref, tgraph.ref, ptr(tperm), ptr(Z), _optr(G), ptr(kstar),
+                                                 _optr(w), _optr(s), K, d, float(beta), one_minus(beta), float(T),
+                                                 int(Z.shape[0]), n_rec, ptr(dZ), _optr(r), _optr(dw), _optr(routed),
+                                                 _optr(graph.hub_scratch(K * d)), _optr(tgraph.hub_scratch(K * d)),
+                                                 int(phase), stream_of(dev)), "dl_factor_bwd_directed_phase")
+
+
+def push_entries(src: torch.Tensor, blocks):
+    """dl_push_entries: for every (dst, src_idx) of `blocks`, dst[t] = src[src_idx[t]] (t < len(src_idx)); dst is
+    a tensor or the device address of a peer's block (same element type as src: 1 or 4 bytes).  One launch."""
+    from ._lib import DlPushDesc
+    if src.element_size() not in (1, 4):
+        raise ValueError("push_entries moves 1- or 4-byte elements")
+    dev = src.device
+    descs = (DlPushDesc * max(len(blocks), 1))()
+    for i, (dst, idx) in enumerate(blocks):
+        if idx.dtype != torch.int32 or idx.device != src.device:
+            raise ValueError("push_entries: source indices must be int32 on the source's device")
+        descs[i].dst = dst.data_ptr() if torch.is_tensor(dst) else dst
+        descs[i].src_idx = idx.data_ptr() if idx.numel() else None
+        descs[i].dst_idx = None
+        descs[i].mask = None
+        descs[i].n = int(idx.numel())
+    with torch.cuda.device(dev):
+        check(lib().dl_push_entries(ptr(src), src.element_size(), descs, len(blocks), stream_of(dev)),
+              "dl_push_entries")
+
+
 class PairBatch:
     """A batch of (u,v) node pairs resident on the GPU (int32 ids), plus -- built lazily, once --
     the node-major incidence lists the atomic-free backward walks.

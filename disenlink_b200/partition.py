@@ -31,6 +31,10 @@ kernels (up to 2048 entries per range; the cuts depend on the local entry count)
 Per step:  push Z -> attention -> need-masks, push s -> aggregation -> push H -> pair scores -> gather prob
            -> loss -> decoder backward -> push dH slices -> backward pass 1 -> push r -> backward pass 2
 
+DirectedPartitionedLinkStep trains on the edge columns as given (no symmetrisation): each rank also holds the
+in-entries of its nodes, the owners of entries push their per-entry records (kstar, w, dw) to the owners of the
+columns (dl_push_entries), and the directed backward runs phase by phase (DESIGN.md section 6a).
+
 The orchestration is backend-agnostic: the product backend (`CudaBackend`) calls the CUDA kernels and the
 exchange goes over peer memory; tests inject a CPU backend and the exchange falls back to torch.distributed
 point-to-point (gloo, world_size 2), which is also the path when the ranks cannot map each other's memory.
@@ -98,6 +102,12 @@ def owned_entries(src: torch.Tensor, dst: torch.Tensor, part: NodePartition):
     rows = torch.cat([src[ms], dst[mt]]) - part.lo
     cols = torch.cat([dst[ms], src[mt]])
     return rows, cols
+
+
+def owned_out_entries(src: torch.Tensor, dst: torch.Tensor, part: NodePartition):
+    """Directed (local_row, global_col) entries whose row this rank owns: the edge columns as given."""
+    m = (src >= part.lo) & (src < part.hi)
+    return src[m] - part.lo, dst[m]
 
 
 def pair_shard(P: int, world: int, rank: int):
@@ -419,6 +429,44 @@ class PeerExchange:
                     arr[recv[q][0]:recv[q][0] + recv[q][1]] = b
         self.barrier()
 
+    def push_entries(self, arr, send, dst_off, recv):
+        """Per-entry records: for every peer q, arr[send[q]] -> the peer's copy of `arr` at dst_off[q] + t
+        (dl_push_entries, one launch).  recv = {q: (first, count)}: what arrives here (torch.distributed path
+        only).  Followed by a barrier."""
+        if self.world == 1:
+            return
+        bases = self.peers.get(id(arr)) if self.available else None
+        if bases is not None:
+            from ._lib import DlPushDesc, check, lib, stream_of
+            peers = [q for q in range(self.world) if q != self.rank]
+            descs = (DlPushDesc * len(peers))()
+            for i, q in enumerate(peers):
+                descs[i].dst = bases[q] + dst_off[q] * arr.element_size()
+                descs[i].src_idx = send[q].data_ptr() if send[q].numel() else None
+                descs[i].dst_idx = None
+                descs[i].mask = None
+                descs[i].n = int(send[q].numel())
+            with torch.cuda.device(self.device):
+                check(lib().dl_push_entries(arr.data_ptr(), arr.element_size(), descs, len(peers),
+                                            stream_of(self.device)), "dl_push_entries")
+        else:
+            ops, bufs = [], {}
+            for q in range(self.world):
+                if q == self.rank:
+                    continue
+                if send[q].numel():
+                    ops.append(dist.P2POp(dist.isend, arr[send[q].long()].contiguous(), q, group=self.group))
+                first, n_in = recv[q]
+                if n_in:
+                    bufs[q] = torch.empty(n_in, dtype=arr.dtype, device=arr.device)
+                    ops.append(dist.P2POp(dist.irecv, bufs[q], q, group=self.group))
+            if ops:
+                for w in dist.batch_isend_irecv(ops):
+                    w.wait()
+            for q, b in bufs.items():
+                arr[recv[q][0]:recv[q][0] + recv[q][1]] = b
+        self.barrier()
+
     def gather_flat(self, full: torch.Tensor, per: int) -> None:
         """All-gather of a flat array split into `world` slices of `per` elements (the P scores)."""
         if self.world == 1:
@@ -451,9 +499,15 @@ class CudaBackend:
 
     def build_csr(self, src, dst, part: NodePartition):
         """-> (rowptr int64 [n_own+1], col int32 [nnz] GLOBAL ids, ascending inside a row)."""
+        return self._csr_of(*owned_entries(src, dst, part), part)
+
+    def build_csr_directed(self, src, dst, part: NodePartition):
+        """build_csr of the edge columns as given (owned out-entries, de-duplicated)."""
+        return self._csr_of(*owned_out_entries(src, dst, part), part)
+
+    def _csr_of(self, rows, cols, part: NodePartition):
         from ._lib import check, lib, ptr, stream_of
-        rows, cols = owned_entries(src, dst, part)
-        dev = src.device
+        dev = rows.device
         E = int(rows.numel())
         L = lib()
         with torch.cuda.device(dev):
@@ -538,6 +592,9 @@ class CudaBackend:
             plan = None
         self.ops.factor_bwd_edges(g, Z, G, kstar, w, s, r, beta, T, dZ, sj=sj, plan=plan)
 
+    def factor_bwd_directed_phase(self, g, gt, tperm, Z, G, kstar, w, s, beta, T, dZ, r, dw, routed, phase):
+        self.ops.factor_bwd_directed_phase(g, gt, tperm, Z, G, kstar, w, s, beta, T, dZ, r, dw, routed, phase)
+
 
 # --------------------------------------------------------------------------------------------
 # the step
@@ -551,16 +608,17 @@ class PartitionedLinkStep:
     `self.H[:n_own]` and all P scores in `self.prob`.
 
     (src, dst) are the edge columns of an undirected graph: the step always trains on their symmetrisation
-    (adj_sym, see owned_entries).  ``directed=True`` -- training on the columns as given -- is refused: the
-    directed backward gathers over the transposed pattern on one GPU (ops.factor_bwd_directed) and has no
-    node-partitioned form."""
+    (adj_sym, see owned_entries).  ``directed=True`` -- training on the columns as given -- is refused here;
+    DirectedPartitionedLinkStep does that."""
+
+    DIRECTED = False
 
     def __init__(self, src, dst, n_global, u, v, labels, weights, K, d, beta, T,
                  world=1, rank=0, group=None, backend=None, device=None, mark=None, balance=True,
                  peer_push=True, bounds=None, directed=False):
-        if directed or getattr(src, "directed", False):
-            raise ValueError("PartitionedLinkStep trains on the symmetrised edge columns only: the directed "
-                             "backward (ops.factor_bwd_directed) runs on one GPU and has no node-partitioned form")
+        if not self.DIRECTED and (directed or getattr(src, "directed", False)):
+            raise ValueError("PartitionedLinkStep trains on the symmetrised edge columns only: use "
+                             "DirectedPartitionedLinkStep to train on directed edge columns as given")
         self.mark = mark if mark is not None else (lambda name: None)  # phase boundary hook (bench)
         self.group = group
         self.be = backend if backend is not None else CudaBackend()
@@ -576,7 +634,7 @@ class PartitionedLinkStep:
                                 else NodePartition(int(n_global), world, rank))
         be = self.be
         # ---- integer setup: CSR of the owned rows, pair shard, incidence lists, halo, local indices ----
-        rowptr, col_g = be.build_csr(src, dst, part)
+        rowptr, col_g = self._build_csr(src, dst, part)
         self.P = int(u.numel())
         self.p_per, self.p_lo, self.p_hi = pair_shard(self.P, world, rank)
         su, sv = u[self.p_lo:self.p_hi].to(torch.int64), v[self.p_lo:self.p_hi].to(torch.int64)
@@ -588,7 +646,7 @@ class PartitionedLinkStep:
             return t[(t < lo) | (t >= hi)]
         if world > 1:
             halo_pair = torch.unique(torch.cat([remote(su), remote(sv), remote(inc_other_g)]))
-            halo_all = torch.unique(torch.cat([remote(col_g), halo_pair]))
+            halo_all = torch.unique(torch.cat([remote(self._read_columns(src, dst, col_g)), halo_pair]))
         else:
             halo_pair = halo_all = torch.empty(0, dtype=torch.int64, device=dev)
         self.plan = plan = HaloPlan(part, halo_all, halo_pair, group)
@@ -599,6 +657,7 @@ class PartitionedLinkStep:
         self.shard = be.make_pairs(plan.to_local(su), plan.to_local(sv), n_tot)
         inc_other_l = plan.to_local(inc_other_g.to(torch.int64)).to(torch.int32) if world > 1 else inc_other_g
         self.inc = be.make_graph(inc_ptr, inc_other_l, n_own, n_tot)
+        n_rec = self._build_records(src, dst, rowptr, col_g)     # per-entry arrays: own entries (+ peers' records)
         del col_g, inc_other_g, su, sv
         # ---- buffers ----
         P_pad = self.p_per * world
@@ -608,8 +667,8 @@ class PartitionedLinkStep:
         self.weights = torch.zeros(P_pad, **f32)
         self.weights[:self.P] = weights
         nnz = self.graph.nnz
-        self.kstar = torch.empty(max(nnz, 1), dtype=torch.uint8, device=dev)
-        self.w = torch.empty(max(nnz, 1), **f32)
+        self.kstar = torch.empty(max(n_rec, 1), dtype=torch.uint8, device=dev)
+        self.w = torch.empty(max(n_rec, 1), **f32)
         # the aggregation gathers slices pre-divided by s (scratch = the dH buffer, idle during the forward;
         # own and halo rows alike: s of the halo has been pushed by then); with DL_F_NO_PRESCALE it gathers
         # s[col, kstar] per entry and hands the per-entry copy to pass 2
@@ -620,7 +679,7 @@ class PartitionedLinkStep:
         self.sj = None if self.prescale else torch.empty(max(nnz, 1), **f32)
         # how pass 1 hands its per-entry dots to pass 2 (and, on one GPU, the symmetric pass 2 with its
         # coefficient scratch); None: pass 2 gathers everything itself (test backend)
-        self.plan_bwd = be.bwd_plan(self.graph, K, d) if hasattr(be, "bwd_plan") else None
+        self.plan_bwd = self._bwd_plan()
         self.Z = torch.zeros(n_tot, K, d, **f32)
         self.Z_own = self.Z[:n_own]
         self.s = torch.ones(n_tot, K, **f32)
@@ -639,7 +698,27 @@ class PartitionedLinkStep:
         self.px = PeerExchange(world, rank, dev, group, enable=peer_push and isinstance(be, CudaBackend))
         self.pushed = False
         if self.px.available:
-            self.pushed = all([self.px.register(t) for t in (self.Z, self.s, self.r, self.H, self.dH, self.prob)])
+            self.pushed = all([self.px.register(t) for t in self._exchanged()])
+
+    # -- what the directed step overrides (DirectedPartitionedLinkStep) --
+    def _build_csr(self, src, dst, part):
+        """-> (rowptr, global columns) of the owned rows: the symmetrised edge columns."""
+        return self.be.build_csr(src, dst, part)
+
+    def _read_columns(self, src, dst, col_g):
+        """Global ids whose Z / s rows the kernels read, besides the pair endpoints."""
+        return col_g
+
+    def _build_records(self, src, dst, rowptr, col_g) -> int:
+        """-> length of the per-entry arrays (kstar, w)."""
+        return self.graph.nnz
+
+    def _bwd_plan(self):
+        return self.be.bwd_plan(self.graph, self.K, self.d) if hasattr(self.be, "bwd_plan") else None
+
+    def _exchanged(self):
+        """The arrays peers write into (registered for peer pushes)."""
+        return (self.Z, self.s, self.r, self.H, self.dH, self.prob)
 
     def close(self):
         """Collective: unmap the peers' buffers (a step object that is rebuilt must not leak mappings)."""
@@ -724,3 +803,178 @@ class PartitionedLinkStep:
         self.forward()
         self.loss_and_grad_logit()
         return self.backward()
+
+
+# --------------------------------------------------------------------------------------------
+# the step on directed edge columns
+# --------------------------------------------------------------------------------------------
+def directed_in_view(src, dst, part: NodePartition, rowptr, col_g):
+    """The in-entries of the owned nodes, from the global edge columns every rank holds.
+
+    rowptr / col_g: this rank's directed CSR (owned rows, GLOBAL columns, ascending in a row).  ->
+      trowptr int64 [n_own+1]   row j - lo lists the in-entries (i, j) of owned node j, by ascending source i
+                                (the order of Graph.transpose_view on one GPU)
+      tsrc    int64 [m]         global source i of every in-entry
+      tperm   int64 [m]         index into the per-entry record space [own CSR entries | tail]: the CSR index of
+                                (i - lo, j) for an owned source, nnz_own + position in the tail otherwise
+      tail_off list [world+1]   the tail = every remote in-entry sorted by (i, j); sender q's block is
+                                [tail_off[q], tail_off[q+1]), in q's own CSR order"""
+    n, lo, hi = part.n_global, part.lo, part.hi
+    dev = col_g.device
+    s64, d64 = src.to(torch.int64), dst.to(torch.int64)
+    m = (d64 >= lo) & (d64 < hi)
+    key = torch.unique((d64[m] - lo) * n + s64[m])                      # sorted: by owned node, then source
+    tj, tsrc = key // n, key % n
+    trowptr = torch.zeros(part.n_local + 1, dtype=torch.int64, device=dev)
+    trowptr[1:] = torch.cumsum(torch.bincount(tj, minlength=part.n_local), 0)
+    entry_key = tsrc * n + tj + lo                                      # (i, j) in global ids
+    own = (tsrc >= lo) & (tsrc < hi)
+    nnz_own = int(col_g.numel())
+    rows = torch.repeat_interleave(torch.arange(part.n_local, device=dev), rowptr[1:] - rowptr[:-1])
+    out_key = (rows + lo) * n + col_g.to(torch.int64)                   # the CSR entries, ascending
+    tail_key = torch.sort(entry_key[~own]).values
+    tperm = torch.empty_like(tsrc)
+    tperm[own] = torch.searchsorted(out_key, entry_key[own])
+    tperm[~own] = nnz_own + torch.searchsorted(tail_key, entry_key[~own])
+    bounds = torch.tensor(part.bounds, dtype=torch.int64, device=dev)
+    tail_off = torch.searchsorted(tail_key // max(n, 1), bounds).tolist()
+    return trowptr, tsrc, tperm, tail_off
+
+
+def entry_send_lists(col_g, part: NodePartition):
+    """-> [world] int64 tensors: the CSR indices of this rank's entries whose column rank q owns, in CSR order (the
+    records q's in-view reads from its tail block for this rank; empty for this rank itself)."""
+    bounds = torch.tensor(part.bounds, dtype=torch.int64, device=col_g.device)
+    owner = torch.searchsorted(bounds[1:], col_g.to(torch.int64), right=True)
+    owner[owner == part.rank] = -1
+    return [torch.nonzero(owner == q).flatten() for q in range(part.world)]
+
+
+class DirectedPartitionedLinkStep(PartitionedLinkStep):
+    """PartitionedLinkStep on the edge columns AS GIVEN: a de-duplicated directed CSR of the owned rows, the
+    directed backward (csrc/bwd_dir.cu) run phase by phase on rank-local graphs.  Same arguments and the same
+    run / forward / loss_and_grad_logit / backward / close contract.
+
+    Entry e = (i, j) lives on the owner of i.  Besides the owned rows each rank holds the IN-VIEW of its nodes
+    (directed_in_view: row j lists the in-entries (i, j), a Graph of its own so in-hubs get hub items) and
+    per-entry records kstar, w, dw of length nnz_own + n_tail: the attention / pass 2 out-side write the own
+    prefix, the owners of remote in-entries push the tail (dl_push_entries).  The halo is the out-neighbours, the
+    in-neighbours and the pair endpoints: the symmetrised graph's halo.
+
+    Per step:  push Z -> attention -> need-masks, push s, push kstar and w records -> aggregation -> push H
+               -> pair scores -> gather prob -> loss -> decoder backward -> push dH slices -> pass 1 (in-view)
+               -> pass 2 out-side -> push dw records -> pass 2 in-side
+    r is read only for the entry's own row, so it is not exchanged."""
+
+    DIRECTED = True
+
+    def _build_csr(self, src, dst, part):
+        return self.be.build_csr_directed(src, dst, part)
+
+    def _read_columns(self, src, dst, col_g):
+        # pass 2's in-side reads Z of the sources of the owned nodes' in-entries
+        d64 = dst.to(torch.int64)
+        m = (d64 >= self.part.lo) & (d64 < self.part.hi)
+        return torch.cat([col_g.to(torch.int64), src.to(torch.int64)[m]])
+
+    def _build_records(self, src, dst, rowptr, col_g) -> int:
+        part, plan, dev = self.part, self.plan, self.device
+        world, rank = part.world, part.rank
+        nnz = self.graph.nnz
+        trowptr, tsrc, tperm, tail_off = directed_in_view(src, dst, part, rowptr, col_g)
+        tcol_l = plan.to_local(tsrc).to(torch.int32) if world > 1 else tsrc.to(torch.int32)
+        self.tgraph = self.be.make_graph(trowptr, tcol_l, self.n_own, self.n_tot)
+        self.tperm = tperm.to(torch.int32)
+        self.n_tail = tail_off[-1] - tail_off[0]
+        if hasattr(self.graph, "_sym"):                         # directed patterns: no symmetric view to try
+            self.graph._sym = False
+            self.tgraph._sym = False
+        sends = entry_send_lists(col_g, part)
+        self.rec_send = [None] * world
+        self.rec_dst = [0] * world
+        self.rec_recv = {q: (nnz + tail_off[q], tail_off[q + 1] - tail_off[q]) for q in range(world)}
+        if world > 1:
+            mine = torch.tensor([nnz] + tail_off, dtype=torch.int64, device=dev)
+            allm = [torch.empty_like(mine) for _ in range(world)]
+            dist.all_gather(allm, mine, group=self.group)
+            for q in range(world):
+                if q == rank:
+                    continue
+                send = sends[q]
+                want = int(allm[q][2 + rank].item()) - int(allm[q][1 + rank].item())
+                if int(send.numel()) != want:
+                    raise RuntimeError(f"rank {rank}: {int(send.numel())} entry records for rank {q}, which expects "
+                                       f"{want} (the ranks disagree on the edge columns)")
+                self.rec_send[q] = send.to(torch.int32)
+                self.rec_dst[q] = int(allm[q][0].item()) + int(allm[q][1 + rank].item())
+        n_rec = nnz + self.n_tail
+        self.dw = torch.empty(max(n_rec, 1), dtype=torch.float32, device=dev)
+        self.routed = torch.empty(max(self.n_own, 1), dtype=torch.int32, device=dev)
+        return n_rec
+
+    def _bwd_plan(self):
+        return None                                             # the directed passes keep no per-entry dots
+
+    def _exchanged(self):
+        return (self.Z, self.s, self.H, self.dH, self.prob, self.kstar, self.w, self.dw)
+
+    def exchange_volume(self):
+        v = super().exchange_volume()
+        n_rec = sum(int(t.numel()) for t in self.rec_send if t is not None)
+        v.update(n_tail=self.n_tail, records_out=n_rec, record_bytes_out_fwd=5 * n_rec, record_bytes_out_bwd=4 * n_rec)
+        return v
+
+    def forward(self):
+        part, be, g, mark, px, plan = self.part, self.be, self.graph, self.mark, self.px, self.plan
+        Z = self.Z
+        mark("begin")
+        # Z halo rows and the record tails: their last readers are the previous step's pass 2 in-side
+        px.barrier()
+        mark("wait")
+        px.push_rows(Z, plan.send_all, plan.recv_all, dst_base=plan.dst_base)
+        mark("ag_Z")
+        be.edge_attn_fwd(g, Z, self.T, self.kstar, self.w, self.s)
+        mark("attn_fwd")
+        if part.world > 1:
+            if hasattr(be, "need_masks"):
+                be.need_masks(g, self.kstar, self.halo_off, part.world, self.masks)
+            px.push_rows(self.s, plan.send_all, plan.recv_all, dst_base=plan.dst_base)
+        mark("ag_s")
+        px.push_entries(self.kstar, self.rec_send, self.rec_dst, self.rec_recv)
+        px.push_entries(self.w, self.rec_send, self.rec_dst, self.rec_recv)
+        mark("ag_rec")
+        be.factor_spmm_fwd(g, Z, self.kstar, self.w, self.s, self.beta, self.H, None,
+                           self.dH if self.prescale else None)
+        mark("spmm_fwd")
+        px.push_rows(self.H, plan.send_pair, plan.recv_pair, dst_idx=plan.dst_pair)
+        mark("ag_H")
+        lo = part.rank * self.p_per
+        if self.p_hi > self.p_lo:
+            be.pair_score_fwd(Z, self.H, self.shard, self.T, self.prob[lo:lo + (self.p_hi - self.p_lo)])
+        mark("pair_fwd")
+        px.gather_flat(self.prob, self.p_per)
+        mark("ag_prob")
+        return self.H, self.prob
+
+    def backward(self):
+        part, be, g, mark, px, plan = self.part, self.be, self.graph, self.mark, self.px, self.plan
+        Z = self.Z
+        be.pair_score_bwd(self.inc, self.inc_pair, Z, self.H, self.dS, self.T, self.dZ, self.dH)
+        mark("pair_bwd")
+        if part.world > 1:
+            # the routed slices G[i, k*] of the peers' in-entries: dl_need_masks on the owned out-entries
+            d4 = self.d // 4 if (self.d % 4 == 0 and (self.d // 4) & (self.d // 4 - 1) == 0) else 0
+            masks = [self.masks[q] for q in range(part.world)] if (d4 and hasattr(be, "need_masks")) else None
+            px.push_rows(self.dH, plan.send_all, plan.recv_all, dst_base=plan.dst_base, masks=masks, vec_per_factor=d4)
+        mark("ag_dH")
+        args = (g, self.tgraph, self.tperm, Z, self.dH, self.kstar, self.w, self.s, self.beta, self.T, self.dZ,
+                self.r, self.dw, self.routed)
+        be.factor_bwd_directed_phase(*args, 1)
+        mark("bwd_gather")
+        be.factor_bwd_directed_phase(*args, 2)
+        mark("bwd_out")
+        px.push_entries(self.dw, self.rec_send, self.rec_dst, self.rec_recv)
+        mark("ag_dw")
+        be.factor_bwd_directed_phase(*args, 3)
+        mark("bwd_in")
+        return self.dZ

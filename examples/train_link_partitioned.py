@@ -6,6 +6,9 @@ across the ranks.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 4 --master-addr 127.0.0.1 --master-port 29533 \\
         examples/train_link_partitioned.py --dataset synthetic --epochs 50
 
+    ... --directed: train on the directed train adjacency (the script's ``adj``, main_disentangled.py:137-140) with
+        disenlink_b200.partition.DirectedPartitionedLinkStep, as examples/train_link.py --directed does on one GPU
+
 Same protocol as the script (85/10/5 split of the edge columns, adjacency = symmetrised train edges, m rounds
 of structured negative sampling on the full edge set, loss = BCE(pos) + BCE(neg)/m over pairs occurring exactly
 once, model selection on validation AUC, test AUC with the best weights).  The validation and test pairs ride in
@@ -27,7 +30,7 @@ import torch
 import torch.distributed as dist
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from disenlink_b200.partition import PartitionedLinkStep  # noqa: E402
+from disenlink_b200.partition import DirectedPartitionedLinkStep, PartitionedLinkStep  # noqa: E402
 
 
 class PartitionedLinkTrainer:
@@ -120,6 +123,7 @@ def main():
     ap.add_argument("--log-every", type=int, default=10)
     ap.add_argument("--locality", action="store_true",
                     help="renumber the nodes with partition.locality_partition first (graphs with locality: smaller halo)")
+    ap.add_argument("--directed", action="store_true", help="train on the directed train adjacency, not adj_sym")
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -146,8 +150,9 @@ def main():
         x, edge_index = order.rows_to_new(x), order.relabel(edge_index)
     edge_index = edge_index.to(device)
     train_edges, u, v, labels, weights, slices = build_pairs(edge_index, n, args.m, args.seed, device)
-    step = PartitionedLinkStep(train_edges[0], train_edges[1], n, u, v, labels, weights, args.nfactor, args.nembed,
-                               args.beta, float(args.temperature), world=world, rank=rank, bounds=bounds)
+    step_cls = DirectedPartitionedLinkStep if args.directed else PartitionedLinkStep
+    step = step_cls(train_edges[0], train_edges[1], n, u, v, labels, weights, args.nfactor, args.nembed,
+                    args.beta, float(args.temperature), world=world, rank=rank, bounds=bounds)
     x_own = x[step.part.lo:step.part.hi].to(device)
     model = Disentangle(x.shape[1], args.nhidden, args.nembed, nfactor=args.nfactor, beta=args.beta,
                         t=args.temperature).to(device)
@@ -165,6 +170,7 @@ def main():
         if rank == 0 and epoch % args.log_every == 0:
             print(f"epoch: {epoch} loss: {float(loss):.5f} val_auc: {best_auc:.4f}", flush=True)
     if rank == 0:
+        print(f"best val auc: {best_auc:.4f}", flush=True)
         print(f"test auc (at the best validation epoch): {best_test:.4f}", flush=True)
     model.load_state_dict(best_state)
     step.close()

@@ -272,6 +272,25 @@ int dl_factor_bwd_directed(const dl_graph* g_host, const dl_graph* gt_host, cons
                            int K, int d, float beta, float one_minus_beta, float T, float* dZ, float* r,
                            float* dw_scratch, uint32_t* routed_scratch, float* hub_ws, float* hub_ws_t,
                            dl_stream_t stream);
+/* One phase of dl_factor_bwd_directed, for the rank-local graphs of a node-partitioned step
+ * (disenlink_b200/partition.py, DirectedPartitionedLinkStep), which exchanges data between the phases:
+ *   phase 1: routed mask of the rows of g, pass 1 over gt (T_, r, dZ += beta G + T_), in-hub finish;
+ *   phase 2: pass 2 out-side over g (writes dw[0, g.nnz)), hub fixup;
+ *   phase 3: pass 2 in-side over gt (reads dw and kstar through tperm), hub fixup.
+ * dl_factor_bwd_directed is phases 1, 2, 3 in order (the same launches).  Rank-local shapes are accepted:
+ * g and gt have the same N (the owned rows) and row_base 0, gt->nnz may differ from g->nnz, every column of
+ * g and gt is below n_tot (the rows of Z, G, s: owned + halo) and every tperm value below n_rec (the length
+ * of the per-entry arrays kstar, w, dw: the own entries [0, g.nnz) followed by records pushed by the owners
+ * of remote in-entries), n_rec >= g->nnz.  Arguments, columns and tperm are checked (DL_EINVAL otherwise);
+ * the index check is one pass over the phase's columns / tperm and one stream synchronisation.
+ * routed_scratch: phase 1 only; r: written by phase 1, read by phase 2; hub_ws: phase 2; hub_ws_t:
+ * phases 1 and 3. */
+int dl_factor_bwd_directed_phase(const dl_graph* g_host, const dl_graph* gt_host, const int32_t* tperm,
+                                 const float* Z, const float* G, const uint8_t* kstar, const float* w,
+                                 const float* s, int K, int d, float beta, float one_minus_beta, float T,
+                                 int64_t n_tot, int64_t n_rec, float* dZ, float* r, float* dw,
+                                 uint32_t* routed_scratch, float* hub_ws, float* hub_ws_t, int phase,
+                                 dl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * (5) factor-weighted link-pair scoring over explicit (u,v) batches.
@@ -429,6 +448,13 @@ typedef struct dl_push_desc {
 } dl_push_desc;
 int dl_push_rows(const void* src, int64_t row_bytes, int vec_per_factor, const dl_push_desc* descs_host,
                  int n_peers, dl_stream_t stream);
+/* dl_push_entries: the per-entry records of the directed step (kstar: 1 byte, w and dw: 4 bytes).  For every
+ * peer q and t in [0, n):  dst_q[(dst_idx ? dst_idx[t] : t)] = src[(src_idx ? src_idx[t] : t)], elements of
+ * elem_bytes (1 or 4) bytes.  dst = the peer's array, already offset to the block that receives this rank's
+ * records; desc.mask must be NULL; a descriptor with n = 0 is allowed.  Plain stores, one launch for all
+ * peers, n_peers <= 15. */
+int dl_push_entries(const void* src, int elem_bytes, const dl_push_desc* descs_host, int n_peers,
+                    dl_stream_t stream);
 /* Which factor slices of an owned row does each peer read?  By the symmetry of adjacency and routing, peer p
  * gathers G[j, k] (j owned here) exactly when this rank holds an entry (j, i) routed to k with i owned by p.
  * masks [n_parts][g.N] (device uint32, overwritten): bit k of masks[p][j] set accordingly.  halo_off
