@@ -220,9 +220,12 @@ def factor_bwd_edges(graph: Graph, Z, G, kstar, w, s, r, beta: float, T: float, 
               "dl_factor_bwd_edges")
 
 
-def factor_bwd(graph: Graph, Z, G, kstar, w, s, beta: float, T: float = 1.0, dZ=None, r=None, sj=None):
+def factor_bwd(graph: Graph, Z, G, kstar, w, s, beta: float, T: float = 1.0, dZ=None, r=None, sj=None,
+               plan: dict = None):
     """dL/dZ through attention + aggregation given G = dL/dH; accumulated into dZ if given.
-    -> (dZ, r).  [ref: autograd of model.py:56-75]"""
+    -> (dZ, r).  `plan` = a bwd_plan(graph, K, d) prepared once and held by the caller (a captured epoch must
+    not query free memory or allocate its scratch per call); None: a new plan per call.
+    [ref: autograd of model.py:56-75]"""
     K, d = _check_Z(Z, graph.n_global)
     Z = Z.contiguous()
     G = G.contiguous()
@@ -232,7 +235,8 @@ def factor_bwd(graph: Graph, Z, G, kstar, w, s, beta: float, T: float = 1.0, dZ=
             dZ = torch.zeros_like(Z)
         if r is None:
             r = torch.empty(graph.n_global, K, dtype=torch.float32, device=dev)
-    plan = bwd_plan(graph, K, d)
+    if plan is None:
+        plan = bwd_plan(graph, K, d)
     factor_bwd_gather(graph, Z, G, kstar, w, s, beta, dZ, r, plan=plan)
     if plan["mode"] == "sym" and not plan["x_valid"]:            # pass 1 took a path without dots: plain pass 2
         plan = None
@@ -270,6 +274,9 @@ def factor_bwd_directed_phase(graph: Graph, tgraph: Graph, tperm, Z, G, kstar, w
     (reads kstar, dw through tperm).  `graph` / `tgraph`: the owned rows and their in-entries (same N, row_base 0),
     columns below Z.shape[0]; kstar, w, dw: the per-entry records [own entries | records of remote in-entries],
     every tperm value below their length.  `routed`: int32 [N] scratch of phase 1."""
+    if torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("dl_factor_bwd_directed_phase checks its indices with a host synchronisation and cannot "
+                           "be captured in a CUDA graph")
     K, d = int(Z.shape[1]), int(Z.shape[2])
     dev = Z.device
     n_rec = min(int(kstar.numel()), int(dw.numel()) if dw is not None else 1 << 62,
@@ -601,7 +608,11 @@ def link_bce_segments(prob, labels, weights, seg_ptr):
 
 def roc_auc(score, labels) -> float:
     """sklearn.metrics.roc_auc_score(labels, score) for binary labels, computed on the device
-    (main_disentangled.py:204,219).  Raises ValueError where sklearn does (one class only, NaN)."""
+    (main_disentangled.py:204,219).  Raises ValueError where sklearn does (one class only, NaN).  Reads the
+    result back to the host, so it refuses to run inside a CUDA graph capture (use roc_auc_stats there)."""
+    if torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("ops.roc_auc returns a host float and cannot be captured in a CUDA graph; "
+                           "use ops.roc_auc_stats / ops.roc_auc_segments, which leave the AUC on the device")
     auc, n_pos, n_neg, n_nan, _ = roc_auc_stats(score, labels).tolist()
     if n_nan:
         raise ValueError("Input contains NaN.")
@@ -616,7 +627,7 @@ class _LinkBCELoss(torch.autograd.Function):
     [ref: model.py:105-114 + main_disentangled.py:195 and its autograd]"""
 
     @staticmethod
-    def forward(ctx, Z, graph, batch, labels, weights, beta, T):
+    def forward(ctx, Z, graph, batch, labels, weights, beta, T, plan):
         Zc = Z.detach().contiguous()
         need_grad = ctx.needs_input_grad[0]        # False under torch.no_grad(): the eager backward is skipped
         if need_grad and not graph.directed:
@@ -634,7 +645,7 @@ class _LinkBCELoss(torch.autograd.Function):
             if graph.directed:
                 factor_bwd_directed(graph, Zc, dH, kstar, w, s, beta, T, dZ=dZ)
             else:
-                factor_bwd(graph, Zc, dH, kstar, w, s, beta, T, dZ=dZ, sj=sj)
+                factor_bwd(graph, Zc, dH, kstar, w, s, beta, T, dZ=dZ, sj=sj, plan=plan)
             ctx.save_for_backward(dZ)
         ctx.mark_non_differentiable(prob, H)
         return loss, prob, H
@@ -644,13 +655,15 @@ class _LinkBCELoss(torch.autograd.Function):
         (dZ,) = ctx.saved_tensors
         # out of place: a second backward through the same graph (retain_graph, accumulation) must see
         # the unscaled dZ again, and the returned gradient must not alias a saved tensor
-        return dZ * gloss, None, None, None, None, None, None
+        return dZ * gloss, None, None, None, None, None, None, None
 
 
-def link_bce_loss(Z, graph: Graph, batch: PairBatch, labels, weights, beta: float, T: float = 1.0):
+def link_bce_loss(Z, graph: Graph, batch: PairBatch, labels, weights, beta: float, T: float = 1.0,
+                  plan: dict = None):
     """sum_p weights[p] * BCE(score(u_p, v_p), labels[p]) with score as in model.py:113.
-    -> (loss, prob [P], H [N,K,d]); differentiable w.r.t. Z only through `loss`."""
-    return _LinkBCELoss.apply(Z, graph, batch, labels, weights, beta, T)
+    -> (loss, prob [P], H [N,K,d]); differentiable w.r.t. Z only through `loss`.  `plan` = a bwd_plan of an
+    undirected graph, passed on to factor_bwd (None: planned per call)."""
+    return _LinkBCELoss.apply(Z, graph, batch, labels, weights, beta, T, plan)
 
 
 def pairs_exactly_once(u, v, n_nodes: int):

@@ -215,10 +215,14 @@ class EarlyStopping:
 
     (a NaN AUC is no improvement).  A stopped run is frozen: its best_auc, stale and snapshot never change
     again, so its result is the one the script's ``break`` gives, while its rows may keep training in the
-    union.  The snapshot starts as the weights given here, which a run that never improves keeps."""
+    union.  The snapshot starts as the weights given here, which a run that never improves keeps.
 
-    def __init__(self, params: Sequence[torch.Tensor], patience: int = 200):
-        self.params = list(params)
+    ``stacked=False`` takes the parameters of one unstacked model (``Disentangle``) as a single run, R = 1:
+    the rule is then ``run()``'s host loop (examples/train_link.py) with its ``deepcopy(state_dict)`` kept on the
+    device, and ``snapshot[i][0]`` is the best copy of ``params[i]``."""
+
+    def __init__(self, params: Sequence[torch.Tensor], patience: int = 200, stacked: bool = True):
+        self.params = list(params) if stacked else [p.detach().unsqueeze(0) for p in params]
         R, dev = int(self.params[0].shape[0]), self.params[0].device
         self.patience = int(patience)
         self.best_auc = torch.zeros(R, dtype=torch.float64, device=dev)

@@ -20,6 +20,11 @@ pattern and its transpose.  Split, negatives and AUC are unchanged.
 one union graph, one stacked model, one optimizer step per epoch (disenlink_b200/runs.py), per-run early
 stopping, then the per-run test AUCs and their mean +- std.  Run r gives what a single run with
 --seed (seed + r) gives, up to the summation order of the batched GEMMs.
+
+--capture E captures the epoch once as a CUDA graph and replays it (disenlink_b200/capture.py): stopping rule and
+model selection on the device, one device-to-host copy per chunk of E epochs, Adam with capturable=True (bias
+correction on the device).  Works with --run R and --directed; the loop ends at the first chunk boundary after
+every run has stopped.
 """
 from __future__ import annotations
 
@@ -34,6 +39,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from disenlink_b200 import data as dl_data  # noqa: E402
 from disenlink_b200 import ops  # noqa: E402
+from disenlink_b200.capture import CapturedEpoch  # noqa: E402
 from disenlink_b200.graph import Graph  # noqa: E402
 from disenlink_b200.model import Disentangle  # noqa: E402
 from disenlink_b200.runs import DisentangleRuns, EarlyStopping, RunSet, edge_labels  # noqa: E402
@@ -94,6 +100,13 @@ def run(args, x, edge_index, device, log=print):
 
     model = Disentangle(x.shape[1], args.nhidden, args.nembed, nfactor=args.nfactor, beta=args.beta,
                         t=args.temperature).to(device)
+    if getattr(args, "capture", None):
+        opt = torch.optim.Adam(model.parameters(), lr=args.lr, weight_decay=5e-4, capturable=True)
+        ce = CapturedEpoch(model, opt, x, graph, train_batch, labels, weights, val_batch, val_lab, test_batch,
+                           test_lab, args.beta, args.temperature, patience=200, chunk=args.capture)
+        out = ce.run(args.epochs, log=log, log_every=args.log_every)
+        log(f"test auc: {out['test_auc'][0]:.4f}")
+        return {"history": out["history"][0], "best_val_auc": out["best_val_auc"][0], "test_auc": out["test_auc"][0]}
     opt = torch.optim.Adam(model.parameters(), lr=args.lr, weight_decay=5e-4)
     best_auc, stale, best_state, history = 0.0, 0, None, []
     for epoch in range(args.epochs):
@@ -158,29 +171,37 @@ def run_batched(args, x, edge_index, device, log=print):
     seeds = [args.seed + r for r in range(args.run)]
     runs = RunSet(edge_index.to(device), n, seeds, args.m, directed=getattr(args, "directed", False))
     model = batched_model(args, x.shape[1], seeds).to(device)
-    opt = torch.optim.Adam(model.parameters(), lr=args.lr, weight_decay=5e-4)
-    stop = EarlyStopping(list(model.parameters()), patience=200)
     R = len(seeds)
-    history = [[] for _ in range(R)]
-    active = [True] * R
-    for epoch in range(args.epochs):
-        host = batched_epoch(args, x, runs, model, opt, stop)
-        for r in range(R):
-            if active[r]:
-                history[r].append((host[r], host[R + r]))
-        active = [not bool(f) for f in host[3 * R:]]
-        if epoch % args.log_every == 0:
-            log(f"epoch: {epoch} active runs: {sum(active)}/{R} loss: {np.mean(host[:R]):.5f} (mean) "
-                f"val_auc: " + " ".join(f"{b:.4f}" for b in host[2 * R:3 * R]))
-        if not any(active):
-            break
-    stop.restore()
-    with torch.no_grad():
-        Z = model.project(x)
-        H = ops.factor_aggregate(Z, runs.graph, args.beta, args.temperature)
-        _, test_prob = ops.pair_score_fwd(Z, H, runs.test, args.temperature, want_logit=False)
-    test_auc = ops.roc_auc_segments(test_prob, runs.test_labels, runs.test_ptr)[:, 0].tolist()
-    best_val = stop.best_auc.tolist()
+    if getattr(args, "capture", None):
+        opt = torch.optim.Adam(model.parameters(), lr=args.lr, weight_decay=5e-4, capturable=True)
+        ce = CapturedEpoch(model, opt, x, runs.graph, runs.train, runs.train_labels, runs.train_weights, runs.val,
+                           runs.val_labels, runs.test, runs.test_labels, args.beta, args.temperature, patience=200,
+                           chunk=args.capture, train_ptr=runs.train_ptr, val_ptr=runs.val_ptr, test_ptr=runs.test_ptr)
+        res = ce.run(args.epochs, log=log, log_every=args.log_every)
+        history, best_val, test_auc = res["history"], res["best_val_auc"], res["test_auc"]
+    else:
+        opt = torch.optim.Adam(model.parameters(), lr=args.lr, weight_decay=5e-4)
+        stop = EarlyStopping(list(model.parameters()), patience=200)
+        history = [[] for _ in range(R)]
+        active = [True] * R
+        for epoch in range(args.epochs):
+            host = batched_epoch(args, x, runs, model, opt, stop)
+            for r in range(R):
+                if active[r]:
+                    history[r].append((host[r], host[R + r]))
+            active = [not bool(f) for f in host[3 * R:]]
+            if epoch % args.log_every == 0:
+                log(f"epoch: {epoch} active runs: {sum(active)}/{R} loss: {np.mean(host[:R]):.5f} (mean) "
+                    f"val_auc: " + " ".join(f"{b:.4f}" for b in host[2 * R:3 * R]))
+            if not any(active):
+                break
+        stop.restore()
+        with torch.no_grad():
+            Z = model.project(x)
+            H = ops.factor_aggregate(Z, runs.graph, args.beta, args.temperature)
+            _, test_prob = ops.pair_score_fwd(Z, H, runs.test, args.temperature, want_logit=False)
+        test_auc = ops.roc_auc_segments(test_prob, runs.test_labels, runs.test_ptr)[:, 0].tolist()
+        best_val = stop.best_auc.tolist()
     out = []
     for r, seed in enumerate(seeds):
         log(f"run {r} (seed {seed}): epochs {len(history[r])} best val auc {best_val[r]:.4f} test auc {test_auc[r]:.4f}")
@@ -190,7 +211,7 @@ def run_batched(args, x, edge_index, device, log=print):
     return {"runs": out, "test_auc_mean": mean, "test_auc_std": std}
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--dataset", default="synthetic")
     ap.add_argument("--root", default="data")
@@ -208,9 +229,18 @@ def main():
     ap.add_argument("--log-every", type=int, default=10)
     ap.add_argument("--directed", action="store_true", help="train on the directed train adjacency, not adj_sym")
     ap.add_argument("--run", type=int, default=1, help="independent runs (seeds --seed + r), trained together")
-    args = ap.parse_args()
+    ap.add_argument("--capture", type=int, default=None, metavar="E",
+                    help="replay the epoch as a CUDA graph, reading the records back every E epochs")
+    args = ap.parse_args(argv)
     if args.run < 1:
         ap.error(f"--run must be >= 1, got {args.run}")
+    if args.capture is not None and args.capture < 1:
+        ap.error(f"--capture must be >= 1 epochs per chunk, got {args.capture}")
+    return args
+
+
+def main():
+    args = parse_args()
     torch.manual_seed(args.seed)
     device = torch.device(f"cuda:{args.gpu}")
     if args.dataset in ("cora", "citeseer", "pubmed"):
