@@ -122,6 +122,10 @@ SIGNATURES = {
     "dl_ipc_open": (_int, [_vp, _vp]),
     "dl_ipc_close": (_int, [_vp]),
     "dl_structured_negative_sampling": (_int, [_GP, _vp, _i64, _i64, _c.c_uint64, _int, _vp, _vp, _vp]),
+    "dl_feat_proj_fwd": (_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _i64, _int, _vp, _i64, _i64, _i64, _vp]),
+    "dl_feat_proj_bwd_workspace_bytes": (_sz, [_i64, _i64, _i64]),
+    "dl_feat_proj_bwd": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _i64, _i64, _i64, _vp, _i64, _i64,
+                                _vp, _i64, _i64, _i64, _i64, _int, _vp, _vp, _vp, _sz, _vp]),
 }
 
 _lib = None

@@ -21,9 +21,9 @@ undone afterwards: weights, optimizer state and stopping state are put back, so 
 Inputs are read by address at every replay: weights loaded in place (``load_state_dict``) are what the next
 replay trains.
 
-Refused before capture (RuntimeError): a sparse ``x``, a row-partitioned graph (the partitioned steps check
-indices with a host synchronisation), and an optimizer that is not capturable (Adam needs ``capturable=True``
-or ``fused=True``).  ``ops.roc_auc`` reads its result on the host and raises inside a capture.
+Refused before capture (RuntimeError): a torch sparse ``x`` (a ``SparseFeatures`` handle is captured), a
+row-partitioned graph (the partitioned steps check indices with a host synchronisation), and an optimizer that
+is not capturable (Adam needs ``capturable=True`` or ``fused=True``).  ``ops.roc_auc`` reads its result on the host and raises inside a capture.
 """
 from __future__ import annotations
 
@@ -33,6 +33,7 @@ from typing import Callable, List, Sequence
 import torch
 
 from . import ops
+from .features import SparseFeatures
 from .graph import Graph
 from .model import Disentangle
 from .runs import DisentangleRuns, EarlyStopping
@@ -71,7 +72,7 @@ class CapturedEpoch:
     union), captured as a CUDA graph (``capture=False``: the same epoch run eagerly, the reference the replay
     is held to).
 
-    x                                  dense features [N, F] on the device
+    x                                  dense features [N, F] on the device, or a features.SparseFeatures handle
     graph                              the train adjacency (adj_sym, or a graph marked directed)
     train, train_labels, train_weights loss pairs; val / val_labels and test / test_labels eval pairs
     train_ptr, val_ptr, test_ptr       the RunSet's int64 [R+1] segment pointers (R > 1 only)
@@ -92,9 +93,9 @@ class CapturedEpoch:
             raise TypeError("CapturedEpoch trains a Disentangle or a DisentangleRuns model")
         if int(chunk) < 1:
             raise ValueError(f"chunk must be >= 1, got {chunk}")
-        if x.layout != torch.strided:
-            raise RuntimeError("CapturedEpoch needs a dense x: the sparse projection (torch.sparse.mm) is not "
-                               "captured; pass x.to_dense()")
+        if not isinstance(x, SparseFeatures) and x.layout != torch.strided:
+            raise RuntimeError("CapturedEpoch needs a dense x or a SparseFeatures handle: the sparse projection "
+                               "(torch.sparse.mm) is not captured; pass x.to_dense() or SparseFeatures.from_sparse(x)")
         if graph.row_base != 0 or graph.n_global != graph.N:
             raise RuntimeError("CapturedEpoch needs a whole graph on one GPU: the row-partitioned steps check "
                                "indices with a host synchronisation and cannot be captured")

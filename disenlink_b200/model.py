@@ -33,6 +33,7 @@ import torch.nn.functional as F
 
 from . import ops
 from ._lib import require_cuda
+from .features import SparseFeatures
 from .graph import Graph
 
 
@@ -314,18 +315,25 @@ class Disentangle(nn.Module):
         self.disentangle_layer1.adjacency = value
         self.disentangle_layer2.adjacency = value
 
-    def project(self, x: torch.Tensor) -> torch.Tensor:
+    def project(self, x: Union[torch.Tensor, SparseFeatures]) -> torch.Tensor:
         """Z [N,K,d] = the K factor MLPs of model.py:106, batched: one [N,F] x [F,K*nhid] GEMM for the
         K first layers (a sparse-dense product when x is a sparse tensor: bag-of-words features are
         ~1 % dense) and one batched [K] x ([N,nhid] x [nhid,d]) product for the second layers, written
         straight into the [N,K,d] layout.  The parameters stay the per-factor nn.Linear modules of
         the reference (same state_dict); the stacked weights are views rebuilt per call, so autograd
         routes the gradients back to them.  Library GEMMs, fp32 -- TF32 would break the 1e-5 parity
-        target."""
+        target.  When x is a ``SparseFeatures`` handle the first layers (with their ReLU) run over its
+        nonzeros in the project's kernels (ops.feature_projection); the second layers are unchanged."""
         K = len(self.factors)
         first = [f.mlp if isinstance(f, Factor) else f.mlp1 for f in self.factors]
-        W1 = torch.cat([m.weight for m in first], dim=0)              # [K*nhid, F]
         b1 = torch.cat([m.bias for m in first], dim=0)
+        if isinstance(x, SparseFeatures):
+            Wt = torch.cat([m.weight.t() for m in first], dim=1)      # [F, K*nhid]
+            hid = ops.feature_projection(x, Wt, b1, relu=not isinstance(self.factors[0], Factor), blocks=K)
+            if isinstance(self.factors[0], Factor):
+                return hid.transpose(0, 1)                            # [N, K, d], contiguous
+            return self._second_layer(hid, False)
+        W1 = torch.cat([m.weight for m in first], dim=0)              # [K*nhid, F]
         tc = self.projection == "3xtf32" and x.is_cuda and x.layout == torch.strided
         if x.is_sparse or x.layout == torch.sparse_csr:
             hid = torch.sparse.mm(x, W1.t()) + b1
@@ -337,6 +345,10 @@ class Disentangle(nn.Module):
         if isinstance(self.factors[0], Factor):
             return hid.view(N, K, -1)
         hid = F.relu(hid).view(N, K, -1).transpose(0, 1)              # [K, N, nhid]
+        return self._second_layer(hid, tc)
+
+    def _second_layer(self, hid: torch.Tensor, tc: bool) -> torch.Tensor:
+        """[K, N, nhid] hidden layers -> Z [N, K, d]."""
         W2 = torch.stack([f.mlp2.weight for f in self.factors], dim=0)  # [K, d, nhid]
         b2 = torch.stack([f.mlp2.bias for f in self.factors], dim=0)    # [K, d]
         if tc:
@@ -345,14 +357,14 @@ class Disentangle(nn.Module):
             Z = torch.baddbmm(b2.unsqueeze(1), hid, W2.transpose(1, 2))   # [K, N, d]
         return Z.transpose(0, 1).contiguous()
 
-    def embed(self, x: torch.Tensor, adj: AdjLike):
+    def embed(self, x: Union[torch.Tensor, SparseFeatures], adj: AdjLike):
         """-> (Z [N,K,d], H [N,K,d], graph)"""
         require_cuda(x, "x")
         Z = self.project(x)
         H, _, _, _, graph = self.disentangle_layer1.sparse_forward(Z, adj)
         return Z, H, graph
 
-    def forward(self, x: torch.Tensor, adj: AdjLike):
+    def forward(self, x: Union[torch.Tensor, SparseFeatures], adj: AdjLike):
         Z, H, graph = self.embed(x, adj)
         N = Z.shape[0]
         T = float(self.temperature)

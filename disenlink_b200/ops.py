@@ -736,3 +736,61 @@ def dense_att(graph: Graph, kstar, w, s, K: int):
         check(lib().dl_dense_att(graph.ref, ptr(kstar), ptr(w), ptr(s), K, ptr(out), stream_of(dev)),
               "dl_dense_att")
     return out
+
+
+# --------------------------------------------------------------------------------------------
+# first layer of the factor MLPs from sparse features (csrc/feat_proj.cu)
+# --------------------------------------------------------------------------------------------
+class _FeatureProjection(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, Wt, b, feats, relu, blocks):
+        F_, J = int(Wt.shape[0]), int(Wt.shape[1])
+        N, nh = feats.N, J // blocks
+        dev = Wt.device
+        with torch.cuda.device(dev):
+            A = torch.empty(N, J, dtype=torch.float32, device=dev)
+            check(lib().dl_feat_proj_fwd(ptr(feats.rowptr), ptr(feats.col), ptr(feats.val), N, F_, ptr(Wt), ptr(b), J,
+                                         int(relu), ptr(A), J, nh, nh, stream_of(dev)), "dl_feat_proj_fwd")
+        out = A.view(N, blocks, nh).transpose(0, 1)               # [blocks, N, nh], the layout the second layer reads
+        ctx.feats, ctx.relu, ctx.shape = feats, bool(relu), (F_, J, nh)
+        ctx.save_for_backward(out)
+        return out
+
+    @staticmethod
+    def backward(ctx, G):
+        (A,) = ctx.saved_tensors
+        feats, (F_, J, nh) = ctx.feats, ctx.shape
+        if G.stride(2) != 1:
+            G = G.contiguous()
+        dev = G.device
+        L = lib()
+        with torch.cuda.device(dev):
+            dWt = torch.empty(F_, J, dtype=torch.float32, device=dev)
+            db = torch.empty(J, dtype=torch.float32, device=dev)
+            ws_bytes = int(L.dl_feat_proj_bwd_workspace_bytes(feats.N, J, feats.n_slots))
+            ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+            check(L.dl_feat_proj_bwd(ptr(feats.row), ptr(feats.cval), ptr(feats.item_col), ptr(feats.item_lo),
+                                     ptr(feats.item_hi), feats.n_items, feats.n_slots, ptr(feats.heavy_col),
+                                     ptr(feats.heavy_ptr), feats.n_heavy, feats.N, F_, ptr(A), A.stride(1),
+                                     A.stride(0), ptr(G), G.stride(1), G.stride(0), nh, J, int(ctx.relu), ptr(dWt),
+                                     ptr(db), ptr(ws), ws_bytes, stream_of(dev)), "dl_feat_proj_bwd")
+        return dWt, db, None, None, None
+
+
+def feature_projection(feats, Wt: torch.Tensor, b: torch.Tensor, relu: bool, blocks: int = 1) -> torch.Tensor:
+    """act(x Wt + b) for x a features.SparseFeatures [N, F], Wt [F, J], b [J]; act = ReLU or the identity.
+    [ref: model.py:24-27,106, the first layer of the K factor MLPs]  -> [blocks, N, J / blocks], the transposed
+    view of a contiguous [N, J] (block k = factor k's hidden layer).  Differentiable w.r.t. Wt and b; the
+    gradient may come back in any layout whose last dimension is contiguous (no copy is made then)."""
+    require_cuda(Wt, "Wt")
+    if not feats.is_cuda or feats.device != Wt.device:
+        raise RuntimeError("the features must be on Wt's CUDA device: disenlink_b200 runs only through its sm_100a "
+                           "CUDA kernels and has no CPU fallback")
+    if Wt.dim() != 2 or Wt.shape[0] != feats.F or Wt.dtype != torch.float32:
+        raise ValueError(f"Wt must be float32 [F={feats.F}, J], got {Wt.dtype} {tuple(Wt.shape)}")
+    J = int(Wt.shape[1])
+    if b.shape != (J,) or b.dtype != torch.float32 or b.device != Wt.device:
+        raise ValueError(f"b must be float32 [{J}] on Wt's device")
+    if blocks < 1 or J % blocks:
+        raise ValueError(f"J = {J} is not a multiple of blocks = {blocks}")
+    return _FeatureProjection.apply(Wt.contiguous(), b.contiguous(), feats, bool(relu), int(blocks))

@@ -24,7 +24,7 @@ nothing, so they are stacked instead of repeated:
 from __future__ import annotations
 
 from collections import OrderedDict
-from typing import List, Sequence
+from typing import List, Sequence, Union
 
 import torch
 import torch.nn as nn
@@ -32,6 +32,7 @@ import torch.nn.functional as F
 
 from . import data, ops
 from ._lib import require_cuda
+from .features import SparseFeatures
 from .graph import Graph
 from .model import Disentangle, Factor2
 
@@ -114,19 +115,24 @@ class DisentangleRuns(nn.Module):
                     raise ValueError(f"{k}: shape {tuple(src.shape)}, expected {tuple(dst.shape)}")
                 dst.copy_(src)
 
-    def project(self, x: torch.Tensor) -> torch.Tensor:
+    def project(self, x: Union[torch.Tensor, SparseFeatures]) -> torch.Tensor:
         """Z [R*N, K, d] of a shared x [N, F]; row r*N + i is run r's node i (Disentangle.project per run).
         The first layers of all runs and factors are one [N,F] x [F, R*K*nhid] GEMM (torch.sparse.mm for a
-        sparse x), the second layers one batched product over the R*K factors.  Library GEMMs, fp32."""
+        sparse x; the project's sparse kernels, ops.feature_projection, for a SparseFeatures x), the second
+        layers one batched product over the R*K factors.  Library GEMMs, fp32."""
         R, K, h, d = self.runs, self.nfactor, self.nhid, self.nembed
         W1 = self.W1.reshape(R * K * h, self.nfeat)
         b1 = self.b1.reshape(R * K * h)
-        if x.is_sparse or x.layout == torch.sparse_csr:
-            hid = torch.sparse.mm(x, W1.t()) + b1
+        if isinstance(x, SparseFeatures):
+            hid = ops.feature_projection(x, W1.t().contiguous(), b1, relu=True, blocks=R * K)   # [R*K, N, nhid]
+            N = x.N
         else:
-            hid = torch.addmm(b1, x, W1.t())                                  # [N, R*K*nhid]
-        N = hid.shape[0]
-        hid = F.relu(hid).view(N, R * K, h).transpose(0, 1)                   # [R*K, N, nhid]
+            if x.is_sparse or x.layout == torch.sparse_csr:
+                hid = torch.sparse.mm(x, W1.t()) + b1
+            else:
+                hid = torch.addmm(b1, x, W1.t())                              # [N, R*K*nhid]
+            N = hid.shape[0]
+            hid = F.relu(hid).view(N, R * K, h).transpose(0, 1)               # [R*K, N, nhid]
         Z = torch.baddbmm(self.b2.reshape(R * K, 1, d), hid, self.W2.reshape(R * K, d, h).transpose(1, 2))
         return Z.view(R, K, N, d).transpose(1, 2).reshape(R * N, K, d)      # [R, N, K, d]
 

@@ -25,6 +25,11 @@ stopping, then the per-run test AUCs and their mean +- std.  Run r gives what a 
 model selection on the device, one device-to-host copy per chunk of E epochs, Adam with capturable=True (bias
 correction on the device).  Works with --run R and --directed; the loop ends at the first chunk boundary after
 every run has stopped.
+
+--sparse-features trains on SparseFeatures.from_dense(x) after the dataset's own preprocessing: the first layer of
+the factor MLPs and its weight gradient run over the nonzeros of x (csrc/feat_proj.cu) instead of a dense SGEMM.
+It pays for the raw bag-of-words features of Cora, Citeseer and Pubmed (about 1 % dense) and not for the
+row-standardised datasets, whose x is dense.  Works with --run R and --capture E.
 """
 from __future__ import annotations
 
@@ -40,6 +45,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from disenlink_b200 import data as dl_data  # noqa: E402
 from disenlink_b200 import ops  # noqa: E402
 from disenlink_b200.capture import CapturedEpoch  # noqa: E402
+from disenlink_b200.features import SparseFeatures  # noqa: E402
 from disenlink_b200.graph import Graph  # noqa: E402
 from disenlink_b200.model import Disentangle  # noqa: E402
 from disenlink_b200.runs import DisentangleRuns, EarlyStopping, RunSet, edge_labels  # noqa: E402
@@ -63,9 +69,16 @@ def synthetic(n=3000, communities=8, deg=12, feat=64, seed=0):
     return x, torch.stack([key // n, key % n]), comm
 
 
+def features(args, x, device):
+    """x as the model takes it: row-standardised where the dataset is (args.standardize), then a SparseFeatures
+    handle with --sparse-features."""
+    x = dl_data.row_standardize(x).to(device) if args.standardize else x.to(device)
+    return SparseFeatures.from_dense(x) if getattr(args, "sparse_features", False) else x
+
+
 def run(args, x, edge_index, device, log=print):
     n = x.shape[0]
-    x = dl_data.row_standardize(x).to(device) if args.standardize else x.to(device)
+    x = features(args, x, device)
     edge_index = edge_index.to(device)
     E = edge_index.shape[1]
     tr, te, va = dl_data.split_edges(E, args.seed, device)
@@ -167,7 +180,7 @@ def run_batched(args, x, edge_index, device, log=print):
     """run() for seeds args.seed + r, r < args.run, trained together (main_disentangled.py:131-224).
     -> {"runs": [{"seed", "history", "best_val_auc", "test_auc"} per run], "test_auc_mean", "test_auc_std"}"""
     n = x.shape[0]
-    x = dl_data.row_standardize(x).to(device) if args.standardize else x.to(device)
+    x = features(args, x, device)
     seeds = [args.seed + r for r in range(args.run)]
     runs = RunSet(edge_index.to(device), n, seeds, args.m, directed=getattr(args, "directed", False))
     model = batched_model(args, x.shape[1], seeds).to(device)
@@ -231,6 +244,10 @@ def parse_args(argv=None):
     ap.add_argument("--run", type=int, default=1, help="independent runs (seeds --seed + r), trained together")
     ap.add_argument("--capture", type=int, default=None, metavar="E",
                     help="replay the epoch as a CUDA graph, reading the records back every E epochs")
+    ap.add_argument("--sparse-features", action="store_true",
+                    help="first layer over the nonzeros of x (SparseFeatures): pays for raw bag-of-words features "
+                         "(cora, citeseer, pubmed), not for the row-standardised datasets, whose x is dense; the "
+                         "default dense SGEMM is the one whose bits match the reference's nn.Linear")
     args = ap.parse_args(argv)
     if args.run < 1:
         ap.error(f"--run must be >= 1, got {args.run}")

@@ -384,6 +384,35 @@ int64_t dl_roc_auc_segments_workspace_bytes(int64_t P, int64_t R);
 int dl_roc_auc_segments(const float* score, const float* labels, int64_t P, const int64_t* seg_ptr, int64_t R,
                         double* out, void* ws, int64_t ws_bytes, dl_stream_t stream);
 
+/* ---- first layer of the factor MLPs from sparse features (csrc/feat_proj.cu) ----------------
+ * [ref: model.py:24-27,106]  A = act(x W1^T + b1) of the K factors (all runs of a union) at once, x [N, F] sparse
+ * bag-of-words features.  x is given as CSR (rowptr int64 [N+1], col int32, val fp32, rows sorted by column) for
+ * the forward and as CSC (row int32, cval fp32, rows ascending inside a column) for the weight gradient.
+ * Wt = W1^T is [F, J] row-major, b [J]; relu = 1: act = ReLU (Factor2), 0: the identity (Factor, nhid == 1).
+ *   forward:   A[n, j] = act( (sum over row n's entries p, in CSR order, of val[p] Wt[col[p], j]) + b[j] )
+ *   backward:  G' = G * 1[A > 0] (relu only);  dWt[f, j] = sum over column f's entries p, in CSC order, of
+ *              cval[p] G'[row[p], j];  db[j] = sum_n G'[n, j].  dWt (contiguous [F, J]) and db are overwritten.
+ * Each sum is one fixed-order chain that depends on neither J nor the launch shape; no atomics, so the results
+ * are bitwise reproducible and a run's block of a union's Wt gives that run's A and dWt on its own.
+ * A and G are addressed as element (n, j) at n * row_stride + (j / blk) * blk_stride + j % blk (blk = nhid,
+ * J % blk == 0): the [B, N, nhid] view of [N, J] the second layer reads and the gradient its backward returns.
+ * The CSC entries are cut into items: items [0, n_slots) are the chunks of the n_heavy columns longer than the
+ * caller's chunk length, in column order, chunks in order (heavy_col [n_heavy], heavy_ptr [n_heavy+1] = their
+ * item ranges); items [n_slots, n_items) are the other columns, one whole (possibly empty) column each.  Item t
+ * covers CSC entries [item_lo[t], item_hi[t]) of column item_col[t]; n_items = F + n_slots - n_heavy.
+ * ws: dl_feat_proj_bwd_workspace_bytes(N, J, n_slots) bytes (G', db partials, chunk partial rows).
+ * Any J >= 1 (float4 access when J, blk, the strides and the pointers allow it).  DL_EINVAL on bad sizes. */
+int dl_feat_proj_fwd(const int64_t* rowptr, const int32_t* col, const float* val, int64_t N, int64_t F,
+                     const float* Wt, const float* b, int64_t J, int relu, float* A, int64_t a_row_stride,
+                     int64_t a_blk_stride, int64_t blk, dl_stream_t stream);
+size_t dl_feat_proj_bwd_workspace_bytes(int64_t N, int64_t J, int64_t n_slots);
+int dl_feat_proj_bwd(const int32_t* row, const float* cval, const int32_t* item_col, const int64_t* item_lo,
+                     const int64_t* item_hi, int64_t n_items, int64_t n_slots, const int32_t* heavy_col,
+                     const int64_t* heavy_ptr, int64_t n_heavy, int64_t N, int64_t F, const float* A,
+                     int64_t a_row_stride, int64_t a_blk_stride, const float* G, int64_t g_row_stride,
+                     int64_t g_blk_stride, int64_t blk, int64_t J, int relu, float* dWt, float* db, void* ws,
+                     size_t ws_bytes, dl_stream_t stream);
+
 /* ---- structured negative sampling ---------------------------------------------------------
  * [ref: main_disentangled.py:160 -- torch_geometric.utils.structured_negative_sampling(edge_index)]
  * For every edge e with source src[e]: k_out[e] ~ U[0, num_nodes) redrawn while (src[e], k) is an
